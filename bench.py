@@ -3,6 +3,7 @@
 1/2/4/8 B200 vs the reference's CPU path, with the HBM roofline fraction of the dominant kernel).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl engine|reference] [--workload c1|c2|c3|c4|c5]
+                  [--dump-outputs DIR]
 
 One "step" = one complete run of the workload from the byte corpus (widen, count, all merges).
   value : merges/s with the corpus already resident in HBM (CUDA events on the engine's stream, max over ranks)
@@ -22,6 +23,9 @@ N > 1 is launched by torch.distributed.run (one rank per GPU); torch.distributed
 
 --impl reference times the UNMODIFIED reference (oracle/_ref/ref_harness, compiled from the reference sources) on
 the host cores, each step a bounded sample of the same workload (first merges of a prefix, scaled; stated in the line).
+
+--dump-outputs DIR writes what the engine's last timed step returned (merge list, ids) as DIR/<name>.npy (see
+dump_outputs()): the corpora are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -58,6 +62,7 @@ WORKLOADS = {
 REF_BIN = os.path.join(ROOT, "oracle/_ref/ref_harness")
 ORACLE_CLI = os.path.join(ROOT, "oracle/_build/bpe_oracle_cli")
 TRAFFIC = os.path.join(ROOT, "profiles", "r2_traffic.json")   # measured dram bytes of the dominant kernel (ncu --set full)
+DUMP_IDS = 1 << 21   # --dump-outputs keeps a fixed sample of this many ids of a longer stream (32 MB with its positions)
 
 
 def peaks():
@@ -352,6 +357,20 @@ def time_training(ctx, M, steps, warmup, world, local, sample_clocks=True):
     return dict(value=merges_done / (dev_ms * 1e-3), dev_ms=dev_ms, wall_ms=wall_ms, clocks=clocks, launches=launches, stats=st)
 
 
+def dump_outputs(out_dir, merges, ids):
+    """Write what a step returned as float64 arrays (exact: ids and positions are below 2^53): merges.npy [k, 2] (training
+    only) and ids.npy.  A stream longer than DUMP_IDS is sampled at fixed positions (seed 0, ascending), which go to
+    ids_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    if merges is not None:
+        np.save(os.path.join(out_dir, "merges.npy"), merges.astype(np.float64))
+    if ids.size > DUMP_IDS:
+        idx = np.sort(np.random.default_rng(0).choice(ids.size, DUMP_IDS, replace=False))
+        np.save(os.path.join(out_dir, "ids_index.npy"), idx.astype(np.float64))
+        ids = ids[idx]
+    np.save(os.path.join(out_dir, "ids.npy"), ids.astype(np.float64))
+
+
 def profiled_roofline(ctx, run, world, shard_bytes, kernel_desc):
     """One extra step with CUDA events around every pass of the dominant kernel."""
     ctx.set_option("profile_replace", 1)
@@ -437,12 +456,16 @@ def bench_engine(args, w, rank, world, local):
         value = n * args.steps / (dev_ms * 1e-3) / 1e9
         metric, unit = "bpe_encode_gb_per_sec", "GB/s"
         final_tokens = st["n_tokens"]
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, None, ctx.download(merges=False)[1])
     else:
         run = lambda: ctx.train(M)
         tt = time_training(ctx, M, args.steps, args.warmup, world, local)
         value, dev_ms, clocks, launches, st = tt["value"], tt["dev_ms"], tt["clocks"], tt["launches"], tt["stats"]
         metric, unit = "bpe_train_merges_per_sec", "merges/s"
         final_tokens = st["n_tokens"]
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, *ctx.download())
 
     # ---- end to end through host buffers (context API, pinned) ---------------------------------------
     nm, nt = ctx.result_sizes()
@@ -460,8 +483,7 @@ def bench_engine(args, w, rank, world, local):
     torch.cuda.synchronize()
     t0 = time.perf_counter()
     e2e_units = 0
-    e2e_steps = max(1, min(args.steps, 3))
-    for _ in range(e2e_steps):
+    for _ in range(args.steps):
         s = e2e_step()
         e2e_units += n / 1e9 if encode_mode else s["n_merges"]
         launches += s["kernel_launches"]
@@ -541,14 +563,14 @@ def bench_engine(args, w, rank, world, local):
             ctx2 = L.Context(local)
             _, s2 = make_shard(w2, 0, 1)
             ctx2.upload_ptr(s2.ctypes.data, s2.size)
-            t2 = time_training(ctx2, w2["merges"], 3, 3, 1, local, sample_clocks=False)
+            t2 = time_training(ctx2, w2["merges"], args.steps, args.warmup, 1, local, sample_clocks=False)
             r2, sp2 = profiled_roofline(ctx2, lambda: ctx2.train(w2["merges"]), 1, s2.size, kdesc)
             if traffic and "c2" in traffic:
                 r2["traffic"] = traffic["c2"].get("dram_bytes_per_launch")
                 r2["traffic_detail"] = traffic["c2"]
             m2, t2ids = ctx2.download()
             g2 = json.load(open(os.path.join(ROOT, "tests", "golden", "c2_full.json")))
-            c2 = {"workload": f"c2: {w2['desc']}", "value": t2["value"], "unit": "merges/s", "ms_per_step": t2["dev_ms"] / 3,
+            c2 = {"workload": f"c2: {w2['desc']}", "value": t2["value"], "unit": "merges/s", "ms_per_step": t2["dev_ms"] / args.steps,
                   "roofline": r2, "equals_oracle_digest": bool(sha(m2) == g2["merges_sha256"] and sha(t2ids) == g2["ids_sha256"])}
             ctx2.close()
             del s2
@@ -608,7 +630,7 @@ def bench_engine(args, w, rank, world, local):
                        else "stream fits in L2 (parity configuration, not a bandwidth one)"},
             "clocks": clocks,
             "e2e": {"value": e2e_value, "unit": unit, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
-                    "ms_per_step": e2e_ms / e2e_steps, "steps": e2e_steps,
+                    "ms_per_step": e2e_ms / args.steps, "steps": args.steps,
                     "path": "bpe_cuda_ctx_upload (pinned host shard) + ctx_train/ctx_encode + ctx_download, per rank"},
             "e2e_paths": e2e_paths,
             "gpu_launches": int(launches),
@@ -634,7 +656,13 @@ def main():
     ap.add_argument("--workload", default=None, choices=list(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="skip the N = 1 extras (c2 block, one-call / drop-in e2e, CPU legs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's merge list and ids to DIR/*.npy "
+                                                          "(--impl engine, --gpus 1)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.impl != "engine" or args.gpus != 1):
+        ap.error("--dump-outputs writes the engine's result on one GPU: it needs --impl engine and --gpus 1")
     if args.workload is None:
         # The 1/2/4/8 curve is asked for on the 1 GB corpus (BASELINE.json configs[2]); it fits one GPU, so every N runs
         # it and the per-N values are comparable.  Config 2 (100 MB, 1 GPU) is measured inside the N = 1 line ("c2").
