@@ -104,6 +104,17 @@ int bpe_cuda_train_file(const char *path, uint64_t max_merges, int n_gpus, bpe_p
 int bpe_cuda_encode_file(const char *path, const bpe_pair_t *merges, size_t n_merges, int n_gpus, uint32_t **tokens_out,
                          size_t *n_tokens, bpe_cuda_stats_t *stats);
 
+/* Encode n_docs documents independently: document i is bytes[offsets[i] .. offsets[i+1]) (offsets: n_docs + 1
+ * non-decreasing values), cut at its first 0x00.  ids of document i = tokens[tok_offsets[i] .. tok_offsets[i+1]),
+ * identical to bpe_cuda_encode() of that document alone.  Device 0; outputs malloc()'d (tok_offsets: n_docs + 1).
+ * One fixed sequence of kernel launches per batch, whatever the number of documents or merges.  Device memory: about
+ * 10 B per input byte (BPE_CUDA_ERR_NOMEM beyond what is free).  A document must be shorter than 4 GiB.  Each document
+ * is encoded by one thread block; one longer than a few hundred KB is slow this way (about 29 s for 4 MB with a
+ * 32,000-merge table on a B200), and bpe_cuda_encode() is the faster path for it. */
+int bpe_cuda_encode_batch(const uint8_t *bytes, const uint64_t *offsets, size_t n_docs, const bpe_pair_t *merges,
+                          size_t n_merges, uint32_t **tokens_out, uint64_t **tok_offsets_out, size_t *n_tokens,
+                          bpe_cuda_stats_t *stats);
+
 void bpe_cuda_free(void *p);
 const char *bpe_cuda_last_error(void);
 int bpe_cuda_device_count(void);
@@ -134,6 +145,14 @@ int bpe_cuda_ctx_truncate(bpe_cuda_ctx_t *ctx, size_t n_shard);
 
 int bpe_cuda_ctx_train(bpe_cuda_ctx_t *ctx, uint64_t max_merges, bpe_cuda_stats_t *stats);
 int bpe_cuda_ctx_encode(bpe_cuda_ctx_t *ctx, const bpe_pair_t *merges, size_t n_merges, bpe_cuda_stats_t *stats);
+
+/* bpe_cuda_encode_batch() on a context, into caller buffers: tokens has room for offsets[n_docs] - offsets[0] ids
+ * (ids <= bytes), tok_offsets for n_docs + 1 values.  Leaves the resident shard and the last train/encode results
+ * untouched.  The pair -> rank table stays on the context and is rebuilt only when the merge list changes, so a
+ * stream of batches with one vocabulary pays for it once. */
+int bpe_cuda_ctx_encode_batch(bpe_cuda_ctx_t *ctx, const uint8_t *bytes, const uint64_t *offsets, size_t n_docs,
+                              const bpe_pair_t *merges, size_t n_merges, uint32_t *tokens, uint64_t *tok_offsets,
+                              bpe_cuda_stats_t *stats);
 
 /* Results of the last train/encode on this context. */
 int bpe_cuda_ctx_result_sizes(bpe_cuda_ctx_t *ctx, size_t *n_merges, size_t *n_tokens_local);

@@ -120,6 +120,45 @@ def encode(data, merges, n_gpus=1):
     return t, st.as_dict()
 
 
+def _as_batch(docs):
+    """docs: a sequence of bytes-like objects, or a (uint8 array, uint64 offsets) tuple -> (bytes, offsets) arrays.
+    Only an offsets array of dtype uint64 selects the tuple form: a tuple of two uint8 documents stays two documents."""
+    if (isinstance(docs, tuple) and len(docs) == 2 and isinstance(docs[0], np.ndarray) and isinstance(docs[1], np.ndarray)
+            and docs[1].dtype == np.uint64):
+        data = _as_bytes_array(docs[0])
+        off = np.ascontiguousarray(docs[1])
+        if off.ndim != 1 or off.size < 1 or int(off[-1]) > data.size:
+            raise ValueError("offsets must be 1-D, hold n_docs + 1 values and end inside the byte array")
+        return data, off
+    parts = [memoryview(d).cast("B") for d in docs]
+    off = np.zeros(len(parts) + 1, dtype=np.uint64)
+    np.cumsum([p.nbytes for p in parts], out=off[1:])
+    return np.frombuffer(b"".join(parts), dtype=np.uint8), off
+
+
+def encode_batch(docs, merges):
+    """Encode every document on its own (each cut at its first NUL) in one call on device 0.
+    -> (ids uint32[m], offsets uint64[n_docs + 1], stats): ids[offsets[i]:offsets[i+1]] == encode(docs[i], merges)."""
+    lib = _lib.load()
+    data, off = _as_batch(docs)
+    mg = np.ascontiguousarray(np.asarray(merges, dtype=np.uint32).reshape(-1, 2))
+    tokens = C.POINTER(C.c_uint32)()
+    toff = C.POINTER(C.c_uint64)()
+    nt = C.c_size_t()
+    st = Stats()
+    rc = lib.bpe_cuda_encode_batch(data.ctypes.data, off.ctypes.data, off.size - 1, mg.ctypes.data, mg.shape[0],
+                                   C.byref(tokens), C.byref(toff), C.byref(nt), C.byref(st))
+    if rc:
+        raise BpeCudaError(rc)
+    try:
+        t = np.ctypeslib.as_array(tokens, shape=(nt.value,)).copy() if nt.value else np.zeros(0, np.uint32)
+        o = np.ctypeslib.as_array(toff, shape=(off.size,)).copy()
+    finally:
+        lib.bpe_cuda_free(tokens)
+        lib.bpe_cuda_free(toff)
+    return t, o, st.as_dict()
+
+
 def decode(tokens, merges):
     """ids -> bytes through the merge list (what decompress() computes, bpe.c:341-394) -> (bytes, stats)."""
     lib = _lib.load()
@@ -200,6 +239,20 @@ class Context:
         if rc:
             raise BpeCudaError(rc)
         return st.as_dict()
+
+    def encode_batch(self, docs, merges):
+        """encode_batch() on this context: the resident shard and the last train/encode results stay as they are, and
+        the pair -> rank table is kept for the next batch with the same merge list."""
+        data, off = _as_batch(docs)
+        mg = np.ascontiguousarray(np.asarray(merges, dtype=np.uint32).reshape(-1, 2))
+        ids = np.empty(max(1, int(off[-1]) - int(off[0])), dtype=np.uint32)   # ids <= bytes
+        toff = np.empty(off.size, dtype=np.uint64)
+        st = Stats()
+        rc = self.lib.bpe_cuda_ctx_encode_batch(self.h, data.ctypes.data, off.ctypes.data, off.size - 1, mg.ctypes.data,
+                                                mg.shape[0], ids.ctypes.data, toff.ctypes.data, C.byref(st))
+        if rc:
+            raise BpeCudaError(rc)
+        return ids[:int(toff[-1])].copy(), toff, st.as_dict()
 
     def decode(self, merges, download=True):
         """Expand this rank's token stream of the last run on the device -> bytes (or their count)."""

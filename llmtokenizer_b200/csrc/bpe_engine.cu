@@ -11,6 +11,7 @@
 #include "bpe_replace.cuh"
 #include "bpe_resolver.cuh"
 #include "bpe_decode.cuh"
+#include "bpe_encode_batch.cuh"
 
 #include <cuda_runtime.h>
 #include <dlfcn.h>
@@ -209,6 +210,24 @@ struct bpe_cuda_ctx
     u32 *d_tile_cnt = nullptr;
     u64 *d_tile_off = nullptr;
     size_t tile_cap = 0;
+    // batch encode (bpe_encode_batch.cuh): buffers of its own, so the resident shard and the last run's results stay
+    uint8_t *d_bb = nullptr;          // the batch's bytes
+    u32 *d_btok = nullptr, *d_brk = nullptr; // per byte: ids at the document's offset / pair ranks; d_brk then holds the
+                                      // compacted ids
+    u64 *d_bdoc = nullptr, *d_btoff = nullptr; // per document: start, then count -> tok_offsets (n_docs + 1)
+    u32 *d_blen = nullptr, *d_border = nullptr;
+    u32 *d_bseg = nullptr, *d_bsegs = nullptr; // global tier: first segment per document; per segment: count, min rank
+    size_t bb_cap = 0, btok_cap = 0, brk_cap = 0, bdoc_cap = 0, btoff_cap = 0, blen_cap = 0, border_cap = 0, bseg_cap = 0,
+           bsegs_cap = 0;
+    u64 *d_rt_key = nullptr;          // pair -> smallest rank (open addressing), kept for the next batch
+    u32 *d_rt_rank = nullptr, *d_bnext = nullptr;
+    size_t rt_key_cap = 0, rt_rank_cap = 0;
+    u32 rt_mask = 0;
+    bool rt_valid = false;
+    std::vector<bpe_pair_t> rt_merges; // the list the table was built from
+    uint2 *d_bmerges = nullptr;
+    size_t bmerges_cap = 0;
+    int cas_grid = 0;                 // persistent CTAs of batch_cascade_kernel (0: not set up yet)
     // communicator (bootstrap + the two collectives of a run's start) and the peer-memory exchange (struct Xchg)
     int rank = 0, world = 1;
     ncclComm_t comm = nullptr;
@@ -1858,6 +1877,10 @@ void bpe_cuda_ctx_destroy(bpe_cuda_ctx_t *c)
     cudaFree(c->d_pos_slot);
     cudaFree(c->d_tile_cnt);
     cudaFree(c->d_tile_off);
+    for (void *p : {(void *)c->d_bb, (void *)c->d_btok, (void *)c->d_brk, (void *)c->d_bdoc, (void *)c->d_btoff,
+                    (void *)c->d_blen, (void *)c->d_border, (void *)c->d_bseg, (void *)c->d_bsegs, (void *)c->d_rt_key, (void *)c->d_rt_rank,
+                    (void *)c->d_bnext, (void *)c->d_bmerges})
+        cudaFree(p);
     if (c->stream)
         cudaStreamDestroy(c->stream);
     delete c;
@@ -2435,6 +2458,322 @@ int bpe_cuda_decode(const uint32_t *tokens, size_t n_tokens, const bpe_pair_t *m
     }
     *bytes_out = out;
     *n_bytes = nb;
+    return 0;
+}
+
+// ---- batch encode (bpe_encode_batch.cuh) ------------------------------------------------------
+// Every argument is checked before any device call, so that a bad call fails the same way with or without a GPU.
+static int batch_check(const uint8_t *bytes, const uint64_t *offsets, size_t n_docs, const bpe_pair_t *merges,
+                       size_t n_merges)
+{
+    if (!offsets || (!merges && n_merges))
+    {
+        set_error("invalid argument: NULL offsets or merges");
+        return BPE_CUDA_ERR_ARG;
+    }
+    if (n_docs >= 0xFFFFFFFFu)
+    {
+        set_error("invalid argument: %zu documents (at most 4,294,967,294 in one batch)", n_docs);
+        return BPE_CUDA_ERR_ARG;
+    }
+    for (size_t i = 0; i < n_docs; i++)
+    {
+        if (offsets[i + 1] < offsets[i])
+        {
+            set_error("invalid argument: offsets[%zu] < offsets[%zu] (offsets must not decrease)", i + 1, i);
+            return BPE_CUDA_ERR_ARG;
+        }
+        if (offsets[i + 1] - offsets[i] >= 0xFFFFFFFFull)
+        {
+            set_error("invalid argument: document %zu is 4 GiB or longer (encode it with bpe_cuda_encode)", i);
+            return BPE_CUDA_ERR_ARG;
+        }
+    }
+    if (!bytes && offsets[n_docs] > offsets[0])
+    {
+        set_error("invalid argument: NULL bytes");
+        return BPE_CUDA_ERR_ARG;
+    }
+    for (size_t r = 0; r < n_merges; r++)
+        if (merges[r].a >= 256 + r || merges[r].b >= 256 + r)
+        {
+            set_error("merge %zu refers to an id that does not exist yet", r);
+            return BPE_CUDA_ERR_ARG;
+        }
+    return 0;
+}
+
+// Encode the batch on the device.  On success the ids are c->d_brk[0 .. *n_tokens) and the offsets c->d_btoff[0 ..
+// n_docs]; stats gets every field but ms_d2h (the caller's copies) and ms_total.
+static int batch_run(bpe_cuda_ctx *c, const uint8_t *bytes, const uint64_t *offsets, size_t n_docs, const bpe_pair_t *merges,
+                     size_t n_merges, size_t *n_tokens, bpe_cuda_stats_t *st)
+{
+    int rc;
+    CU(cudaSetDevice(c->device));
+    memset(st, 0, sizeof *st);
+    const u64 base = offsets[0], N = offsets[n_docs] - base;
+    // lengths after the NUL cut; work order: longest first among the documents of the block and global tiers (an exact
+    // sort for the global tier, 64-byte buckets below it: O(n_docs)), then the warp tier in input order
+    std::vector<u64> doc(n_docs);
+    std::vector<u32> len(n_docs), order;
+    order.reserve(n_docs);
+    u64 n_input = 0;
+    std::vector<u32> global_docs;
+    std::vector<u32> bucket_cnt(BLOCK_CAP / 64 + 2, 0);
+    for (size_t i = 0; i < n_docs; i++)
+    {
+        const uint8_t *p = bytes + offsets[i];
+        const size_t span = offsets[i + 1] - offsets[i];
+        const void *nul = span ? memchr(p, 0, span) : nullptr;
+        doc[i] = offsets[i] - base;
+        len[i] = (u32)(nul ? (const uint8_t *)nul - p : span);
+        n_input += len[i];
+        if (len[i] > BLOCK_CAP)
+            global_docs.push_back((u32)i);
+        else if (len[i] > WARP_CAP)
+            bucket_cnt[len[i] / 64]++;
+    }
+    std::sort(global_docs.begin(), global_docs.end(), [&](u32 x, u32 y) { return len[x] > len[y] || (len[x] == len[y] && x < y); });
+    order = global_docs;
+    {
+        std::vector<u32> start(bucket_cnt.size());
+        u32 acc = (u32)order.size();
+        for (size_t b = bucket_cnt.size(); b-- > 0;)
+        {
+            start[b] = acc;
+            acc += bucket_cnt[b];
+        }
+        order.resize(acc);
+        for (size_t i = 0; i < n_docs; i++)
+            if (len[i] > WARP_CAP && len[i] <= BLOCK_CAP)
+                order[start[len[i] / 64]++] = (u32)i;
+    }
+    const u32 n_big = (u32)order.size();
+    for (size_t i = 0; i < n_docs; i++)
+        if (len[i] <= WARP_CAP)
+            order.push_back((u32)i);
+    // global tier: segments of SEG positions per document (cascade_segmented)
+    std::vector<u32> seg_base(n_docs, 0);
+    size_t n_segs = 0;
+    for (u32 i : global_docs)
+    {
+        seg_base[i] = (u32)n_segs;
+        n_segs += (len[i] + SEG - 1) / SEG;
+    }
+    // device memory: 9 B per input byte (bytes, ids, ranks) + 32 B per document + 8 B per 4 KB segment + the rank
+    // table, each buffer with the 1/8 headroom dec_reserve() gives it
+    size_t rt_cap = 64; // a power of two, at least twice the merges: short probe chains
+    while (rt_cap < 2 * n_merges)
+        rt_cap <<= 1;
+    {
+        size_t free_b = 0, total_b = 0;
+        CU(cudaMemGetInfo(&free_b, &total_b));
+        auto grown = [](size_t n) { return n + n / 8 + 256; };
+        const size_t have = c->bb_cap + 4 * (c->btok_cap + c->brk_cap) + 8 * (c->bdoc_cap + c->btoff_cap) +
+                            4 * (c->blen_cap + c->border_cap + c->bseg_cap + c->bsegs_cap);
+        const size_t need = grown((size_t)N + 16) + 8 * grown((size_t)N + 1) + 16 * grown(n_docs + 1) +
+                            12 * grown(n_docs + 1) + 4 * grown(2 * n_segs + 1) + 12 * rt_cap + (64u << 20);
+        if (need > free_b + have)
+        {
+            set_error("batch of %llu bytes needs about %zu MB of device memory (about 10 B per input byte), %zu MB are free",
+                      (unsigned long long)N, need >> 20, (free_b + have) >> 20);
+            return BPE_CUDA_ERR_NOMEM;
+        }
+    }
+    if ((rc = dec_reserve(c->d_bb, c->bb_cap, (size_t)N + 16)) || (rc = dec_reserve(c->d_btok, c->btok_cap, (size_t)N + 1)) ||
+        (rc = dec_reserve(c->d_brk, c->brk_cap, (size_t)N + 1)) || (rc = dec_reserve(c->d_bdoc, c->bdoc_cap, n_docs + 1)) ||
+        (rc = dec_reserve(c->d_btoff, c->btoff_cap, n_docs + 1)) || (rc = dec_reserve(c->d_blen, c->blen_cap, n_docs + 1)) ||
+        (rc = dec_reserve(c->d_border, c->border_cap, n_docs + 1)) || (rc = dec_reserve(c->d_bseg, c->bseg_cap, n_docs + 1)) ||
+        (rc = dec_reserve(c->d_bsegs, c->bsegs_cap, 2 * n_segs + 1)))
+        return rc;
+    if (!c->d_bnext)
+        CU(cudaMalloc(&c->d_bnext, sizeof(u32)));
+    if (!c->cas_grid)
+    {
+        CU(cudaFuncSetAttribute(batch_cascade_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CAS_SMEM_BYTES));
+        int occ = 0;
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, batch_cascade_kernel, CAS_THREADS, CAS_SMEM_BYTES));
+        c->cas_grid = c->sm_count * std::max(1, occ);
+    }
+    {
+        const auto h0 = std::chrono::steady_clock::now();
+        if (N)
+            CU(cudaMemcpyAsync(c->d_bb, bytes + base, N, cudaMemcpyHostToDevice, c->stream));
+        if (n_docs)
+        {
+            CU(cudaMemcpyAsync(c->d_bdoc, doc.data(), n_docs * sizeof(u64), cudaMemcpyHostToDevice, c->stream));
+            CU(cudaMemcpyAsync(c->d_blen, len.data(), n_docs * sizeof(u32), cudaMemcpyHostToDevice, c->stream));
+            CU(cudaMemcpyAsync(c->d_border, order.data(), n_docs * sizeof(u32), cudaMemcpyHostToDevice, c->stream));
+            CU(cudaMemcpyAsync(c->d_bseg, seg_base.data(), n_docs * sizeof(u32), cudaMemcpyHostToDevice, c->stream));
+        }
+        CU(cudaStreamSynchronize(c->stream));
+        st->ms_h2d = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - h0).count();
+    }
+    cudaEvent_t ev[2] = {nullptr, nullptr};
+    CU(cudaEventCreate(&ev[0]));
+    if (cudaEventCreate(&ev[1]) != cudaSuccess)
+    {
+        cudaEventDestroy(ev[0]);
+        set_error("cudaEventCreate failed");
+        return BPE_CUDA_ERR_CUDA;
+    }
+    struct EvGuard
+    {
+        cudaEvent_t *e;
+        ~EvGuard()
+        {
+            cudaEventDestroy(e[0]);
+            cudaEventDestroy(e[1]);
+        }
+    } ev_guard{ev};
+    u64 launches = 0;
+    CU(cudaEventRecord(ev[0], c->stream));
+    // the rank table: rebuilt only when the merge list differs from the one it was built from
+    const bool rebuild = !c->rt_valid || c->rt_merges.size() != n_merges ||
+                         (n_merges && memcmp(c->rt_merges.data(), merges, n_merges * sizeof(bpe_pair_t)));
+    if (rebuild)
+    {
+        c->rt_valid = false; // until the batch that builds it has completed
+        if ((rc = dec_reserve(c->d_rt_key, c->rt_key_cap, rt_cap)) || (rc = dec_reserve(c->d_rt_rank, c->rt_rank_cap, rt_cap)) ||
+            (rc = dec_reserve(c->d_bmerges, c->bmerges_cap, n_merges + 1)))
+            return rc;
+        c->rt_mask = (u32)(rt_cap - 1);
+        CU(cudaMemsetAsync(c->d_rt_key, 0xFF, rt_cap * sizeof(u64), c->stream));
+        CU(cudaMemsetAsync(c->d_rt_rank, 0xFF, rt_cap * sizeof(u32), c->stream));
+        if (n_merges)
+            CU(cudaMemcpyAsync(c->d_bmerges, merges, n_merges * sizeof(bpe_pair_t), cudaMemcpyHostToDevice, c->stream));
+        const int grid = (int)std::max<size_t>(1, std::min<size_t>((n_merges + 255) / 256, (size_t)c->sm_count * 4));
+        batch_rank_table_kernel<<<grid, 256, 0, c->stream>>>(c->d_bmerges, (u32)n_merges, c->d_rt_key, c->d_rt_rank, c->rt_mask);
+        launches++;
+    }
+    CasArgs a;
+    a.bytes = c->d_bb;
+    a.doc_off = c->d_bdoc;
+    a.doc_len = c->d_blen;
+    a.order = c->d_border;
+    a.n_docs = (u32)n_docs;
+    a.n_big = n_big;
+    a.n_items = n_big + (u32)((n_docs - n_big + CAS_WARPS - 1) / CAS_WARPS);
+    a.tok = c->d_btok;
+    a.rk = c->d_brk;
+    a.seg_base = c->d_bseg;
+    a.seg_cnt = c->d_bsegs;
+    a.seg_min = c->d_bsegs + n_segs;
+    a.count = c->d_btoff;
+    a.next_item = c->d_bnext;
+    a.rt = RankTable{c->d_rt_key, c->d_rt_rank, c->rt_mask};
+    CU(cudaMemsetAsync(c->d_bnext, 0, sizeof(u32), c->stream));
+    batch_cascade_kernel<<<c->cas_grid, CAS_THREADS, CAS_SMEM_BYTES, c->stream>>>(a);
+    decode_scan_kernel<<<1, 1024, 0, c->stream>>>(c->d_btoff, n_docs);
+    batch_gather_kernel<<<c->sm_count * 8, 256, 0, c->stream>>>(c->d_btok, c->d_bdoc, c->d_btoff, (u32)n_docs, c->d_brk);
+    launches += 3;
+    CU(cudaGetLastError());
+    CU(cudaEventRecord(ev[1], c->stream));
+    u64 m = 0;
+    CU(cudaMemcpyAsync(&m, c->d_btoff + n_docs, sizeof m, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    float ms = 0;
+    CU(cudaEventElapsedTime(&ms, ev[0], ev[1]));
+    if (rebuild)
+    {
+        c->rt_merges.assign(merges, merges + n_merges);
+        c->rt_valid = true;
+    }
+    st->n_input = n_input;
+    st->n_merges = n_merges;
+    st->n_tokens = m;
+    st->kernel_launches = launches;
+    st->ms_device = ms;
+    *n_tokens = (size_t)m;
+    return 0;
+}
+
+int bpe_cuda_ctx_encode_batch(bpe_cuda_ctx_t *c, const uint8_t *bytes, const uint64_t *offsets, size_t n_docs,
+                              const bpe_pair_t *merges, size_t n_merges, uint32_t *tokens, uint64_t *tok_offsets,
+                              bpe_cuda_stats_t *stats)
+{
+    if (!c || !tok_offsets || (!tokens && offsets && offsets[n_docs] > offsets[0]))
+    {
+        set_error("invalid argument: NULL context or output buffer");
+        return BPE_CUDA_ERR_ARG;
+    }
+    int rc = batch_check(bytes, offsets, n_docs, merges, n_merges);
+    if (rc)
+        return rc;
+    const auto t0 = std::chrono::steady_clock::now();
+    bpe_cuda_stats_t st;
+    size_t m = 0;
+    if ((rc = batch_run(c, bytes, offsets, n_docs, merges, n_merges, &m, &st)))
+        return rc;
+    const auto h0 = std::chrono::steady_clock::now();
+    CU(cudaMemcpyAsync(tok_offsets, c->d_btoff, (n_docs + 1) * sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    if (m && (rc = download_staged(c, tokens, c->d_brk, m * sizeof(u32))))
+        return rc;
+    const auto t1 = std::chrono::steady_clock::now();
+    st.ms_d2h = std::chrono::duration<double, std::milli>(t1 - h0).count();
+    st.ms_total = std::chrono::duration<double, std::milli>(t1 - t0).count();
+    if (stats)
+        *stats = st;
+    return 0;
+}
+
+int bpe_cuda_encode_batch(const uint8_t *bytes, const uint64_t *offsets, size_t n_docs, const bpe_pair_t *merges,
+                          size_t n_merges, uint32_t **tokens_out, uint64_t **tok_offsets_out, size_t *n_tokens,
+                          bpe_cuda_stats_t *stats)
+{
+    if (!tokens_out || !tok_offsets_out || !n_tokens)
+    {
+        set_error("invalid argument: NULL output pointer");
+        return BPE_CUDA_ERR_ARG;
+    }
+    *tokens_out = nullptr;
+    *tok_offsets_out = nullptr;
+    *n_tokens = 0;
+    int rc = batch_check(bytes, offsets, n_docs, merges, n_merges);
+    if (rc)
+        return rc;
+    const auto t0 = std::chrono::steady_clock::now();
+    bpe_cuda_ctx_t *c = nullptr;
+    if ((rc = bpe_cuda_ctx_create(0, &c)))
+        return rc;
+    bpe_cuda_stats_t st;
+    size_t m = 0;
+    uint32_t *tok = nullptr;
+    uint64_t *toff = nullptr;
+    auto body = [&]() -> int {
+        int r = batch_run(c, bytes, offsets, n_docs, merges, n_merges, &m, &st);
+        if (r)
+            return r;
+        tok = (uint32_t *)malloc(std::max<size_t>(1, m) * sizeof(uint32_t));
+        toff = (uint64_t *)malloc((n_docs + 1) * sizeof(uint64_t));
+        if (!tok || !toff)
+        {
+            set_error("out of host memory");
+            return BPE_CUDA_ERR_NOMEM;
+        }
+        const auto h0 = std::chrono::steady_clock::now();
+        CU(cudaMemcpyAsync(toff, c->d_btoff, (n_docs + 1) * sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+        if (m && (r = download_staged(c, tok, c->d_brk, m * sizeof(u32))))
+            return r;
+        st.ms_d2h = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - h0).count();
+        return 0;
+    };
+    rc = body();
+    bpe_cuda_ctx_destroy(c);
+    if (rc)
+    {
+        free(tok);
+        free(toff);
+        return rc;
+    }
+    st.ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats)
+        *stats = st;
+    *tokens_out = tok;
+    *tok_offsets_out = toff;
+    *n_tokens = m;
     return 0;
 }
 
