@@ -175,8 +175,8 @@ int bpe_cuda_ctx_decode_compare(bpe_cuda_ctx_t *ctx, uint64_t *n_diff);
 const uint8_t *bpe_cuda_ctx_device_decoded(bpe_cuda_ctx_t *ctx);
 
 /* knobs: "profile_replace" (0/1), "batch_steps" (merge steps enqueued per host poll),
- * "smem_hist_max_vocab", "force_census" (0/1), "batch_max" (merges per pass, 1 = off), "batch_min_z",
- * "inplace" (0/1), "ranges", "pdl" (0/1), "speculate" (0/1), "use_stream" (0/1).  Returns 0 if the knob exists. */
+ * "smem_hist_max_vocab", "batch_max" (merges per pass, 1 = off), "batch_min_z", "ranges",
+ * "xchg_cap" (initial entries per inbox slot).  Returns 0 if the knob exists. */
 int bpe_cuda_ctx_set_option(bpe_cuda_ctx_t *ctx, const char *name, long long value);
 
 #ifdef __cplusplus

@@ -141,8 +141,6 @@ struct bpe_cuda_ctx
     DevState *h_st = nullptr;              // the latest copy of the control block (one of h_buf)
     DevState *h_buf[2] = {nullptr, nullptr}; // pinned
     cudaEvent_t poll_ev[2] = {nullptr, nullptr};
-    int pdl = 1;                             // programmatic dependent launch between the step kernels
-    int speculate = 1;                       // enqueue the next batch before the current one has been polled
     // ranged layout: per buffer, length and edge tokens of every range
     u32 *d_rcnt[2] = {nullptr, nullptr};
     u32 *d_redge[2] = {nullptr, nullptr};
@@ -154,7 +152,7 @@ struct bpe_cuda_ctx
     // delta vectors (+ edge-record header)
     int32_t *d_delta = nullptr;
     size_t delta_cap = 0;
-    // pair table (+ per-segment maxima of the hierarchical argmax)
+    // pair table
     u64 *d_tkey = nullptr, *d_tmeta = nullptr;
     u64 tcap = 0;
     u32 *d_cflag = nullptr;  // candidate-membership bit per table slot
@@ -165,23 +163,16 @@ struct bpe_cuda_ctx
         u64 cap = 0;
     } arena[2];
     int arena_cur = 0;
-    int inplace = 1;              // RANGED passes compact the stream inside its own buffer (half the working set: late
-                                  // streams stay in the 126 MB L2 from pass to pass); BPE_CUDA_INPLACE=0 ping-pongs
-    int l2_pin = 0;               // keep the pair table in L2 (access policy window); measured: no gain for apply/select and
-                                  // 25 % slower passes on B200, so off (BPE_CUDA_L2_PIN=1 turns it on)
-    size_t l2_window_max = 0, l2_persist_bytes = 0;
     double host_ms[6] = {0, 0, 0, 0, 0, 0}; // wall clock of host-side phases (debug): rehash, candidates, pause, poll wait, enqueue, setup
     u32 *d_cand = nullptr;   // candidate slots of the argmax (fixed capacity)
-    u32 *d_touched = nullptr; // delta counters touched by the current pass
     SelPart *d_part = nullptr;
     u32 cand_T = 0;          // host copy of the list threshold we asked for (0 = whole-table selection)
     int batch_max = BATCH_MAX; // merges per pass (1 = off)
     int batch_min_z = -1;      // (-1: where the shared-memory delta histogram ends)
-    int pad_unused_bz = 0;       // first id from which merges may share a pass
     bool run_encode = false;   // the current run applies a given merge list
     u64 run_max_merges = 0;    // its merge cap (0 = none)
     int ranges_opt = 0;      // test knob: number of ranges (0 = two per SM)
-    int want_ranged = 0;     // this run uses the streaming kernel (RANGED layout) for its a != b passes
+    int want_ranged = 0;     // this run uses the streaming kernel (RANGED layout) for its passes
     u32 list_retry_below = ~0u; // whole-table mode: try a list again once the best count is below this
     bool fresh_select = false;  // the candidate list ran empty: one whole-table selection must say what the maximum is now
                                 // before any new list is chosen (the control block's `freq` is stale until then)
@@ -251,8 +242,6 @@ struct bpe_cuda_ctx
     int smem_hist_max_vocab = 448;  // ids below this: one merge per pass, deltas privatised in shared memory (7 KB); above: batched
                                     // passes with global RED.  Measured on config 2 (final batching rules): 320 -> 138.8 ms,
                                     // 448 -> 137.3, 512 -> 139.3, 640 -> 141.8 (with the first rules: 1792 -> 209, 640 -> 182)
-    int force_census = 0;
-    int use_stream = 1;
     int replace_occ[2] = {0, 0};
     int stream_occ[2] = {0, 0}; // CTAs per SM of replace_stream_kernel<false>, <true> at the largest histogram
     // profiling events
@@ -489,7 +478,6 @@ static int ensure_logs(bpe_cuda_ctx *c, size_t merges)
 }
 
 constexpr u32 CAND_CAP = 65536;
-constexpr u32 TOUCHED_CAP = 1u << 20;
 
 // Pair-table memory comes from two arenas that only ever grow and live as long as the context: a
 // rehash builds the new table in the arena the current one does not use.  (cudaMalloc / cudaFree
@@ -514,24 +502,6 @@ static int table_alloc(bpe_cuda_ctx *c, u64 cap, int arena)
     return 0;
 }
 
-// Ask for the live table (keys + counts) to be kept in L2 across the streaming passes: the apply / select
-// kernels are chains of dependent accesses to it, and every pass would otherwise evict it.
-static void table_pin_l2(bpe_cuda_ctx *c, int arena, u64 cap)
-{
-    if (!c->l2_pin || c->l2_window_max == 0)
-        return;
-    cudaStreamAttrValue v;
-    memset(&v, 0, sizeof v);
-    const size_t bytes = std::min<size_t>((size_t)cap * 2 * sizeof(u64), (size_t)c->l2_window_max);
-    v.accessPolicyWindow.base_ptr = c->arena[arena].key;
-    v.accessPolicyWindow.num_bytes = bytes;
-    v.accessPolicyWindow.hitRatio = std::min(1.0f, (float)((double)c->l2_persist_bytes / (double)bytes));
-    v.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-    v.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-    if (cudaStreamSetAttribute(c->stream, cudaStreamAttributeAccessPolicyWindow, &v) != cudaSuccess)
-        cudaGetLastError(); // a hint only
-}
-
 static void table_free(bpe_cuda_ctx *c)
 {
     for (int i = 0; i < 2; i++)
@@ -550,7 +520,6 @@ static void table_adopt(bpe_cuda_ctx *c, int arena, u64 cap)
     c->d_tmeta = c->arena[arena].meta;
     c->d_cflag = c->arena[arena].cflag;
     c->tcap = cap;
-    table_pin_l2(c, arena, cap);
 }
 
 static int table_rehash(bpe_cuda_ctx *c, u64 new_cap)
@@ -684,7 +653,7 @@ static cudaError_t launch_chained(bpe_cuda_ctx *c, void (*kernel)(KArgs...), int
     cfg.stream = c->stream;
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = c->pdl ? 1 : 0;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at;
     cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
@@ -712,7 +681,7 @@ static int pos_grid(bpe_cuda_ctx *c, u64 n) { return (int)std::max<u64>(1, std::
 static int enqueue_census(bpe_cuda_ctx *c, u64 n_upper, int resolver)
 {
     const int g = pos_grid(c, n_upper);
-    census_begin_kernel<<<1, 1, 0, c->stream>>>(c->d_st, c->d_rs, resolver, c->force_census);
+    census_begin_kernel<<<1, 1, 0, c->stream>>>(c->d_st, c->d_rs, resolver);
     census_mark_kernel<<<g, 256, 0, c->stream>>>(c->d_st, c->d_rs, c->d_first, c->d_pos_slot);
     census_count_kernel<<<g, 256, 0, c->stream>>>(c->d_st, c->d_rs, c->d_first, c->d_pos_slot);
     census_update_kernel<<<1, 1, 0, c->stream>>>(c->d_st, c->d_rs);
@@ -844,7 +813,7 @@ static int enqueue_step(bpe_cuda_ctx *c, u32 z, u64 n_upper, bool encode, bool c
     const bool hist = ((int)z + 1 <= c->smem_hist_max_vocab);
     if (ranged)
     {
-        // RANGED stream, a != b: one CTA per range, no dependency between CTAs (a == b pauses the loop instead)
+        // RANGED stream: one CTA per range (a == b runs same_pair_range inside the same kernel)
         // the histogram always gets its full budget: the device may be ahead of this id estimate, or batch merges
         const size_t vsmem = stream_smem_bytes(hist, hist ? (u32)c->smem_hist_max_vocab - 1 : 0);
         if (hist)
@@ -1077,9 +1046,7 @@ static int run_loop(bpe_cuda_ctx *c, bool encode)
         const bool stat = (sharded(c) ? h->n_global : h->n) < STATIC_LIMIT;
         if (!encode && !sharded(c))
         {
-            if (c->force_census)
-                X.census = true;
-            else if (stat)
+            if (stat)
             {
                 const u64 dmax = (u64)h->distinct + X.margin;
                 for (int t = 0; t < REF_THREADS; t++)
@@ -1123,7 +1090,7 @@ static int run_loop(bpe_cuda_ctx *c, bool encode)
             Y.n_upper = X.n_upper;
             Y.census = false;
             Y.ranged = X.ranged;
-            const bool spec = c->speculate && Y.G > 0 && !X.census && !stat && !prev->static_mode &&
+            const bool spec = Y.G > 0 && !X.census && !stat && !prev->static_mode &&
                               (encode || prev->n_global >= STATIC_LIMIT) &&
                               occ_bound + Y.margin <= c->tcap / 2 + c->tcap / 8 &&
                               delta_need(c, z_ub + Y.G * bm + 2) <= c->delta_cap && m_ub + Y.G * bm + 2 <= c->merges_cap;
@@ -1169,7 +1136,7 @@ static int run_loop(bpe_cuda_ctx *c, bool encode)
 }
 
 // ---------------------------------------------------------------------------------------------
-static int init_state(bpe_cuda_ctx *c, u64 n_local, u64 max_merges, bool encode, size_t enc_total)
+static int init_state(bpe_cuda_ctx *c, u64 n_local, u64 max_merges, size_t enc_total)
 {
     DevState s;
     memset(&s, 0, sizeof s);
@@ -1177,7 +1144,6 @@ static int init_state(bpe_cuda_ctx *c, u64 n_local, u64 max_merges, bool encode,
     s.tok[1] = c->d_tok_alloc[1] + 4;
     s.tok_real[0] = s.tok[0];
     s.tok_real[1] = s.tok[1];
-    s.inplace = (u32)c->inplace;
     s.cur = 0;
     s.epoch = 1;
     s.n = n_local;
@@ -1186,9 +1152,6 @@ static int init_state(bpe_cuda_ctx *c, u64 n_local, u64 max_merges, bool encode,
     s.tkey = c->d_tkey;
     s.tmeta = c->d_tmeta;
     s.tcap = c->tcap;
-    s.touched = c->d_touched;
-    s.touched_cap = TOUCHED_CAP;
-    s.use_touched = 0;
     s.cand = c->d_cand;
     s.cflag = c->d_cflag;
     s.cand_cap = CAND_CAP;
@@ -1207,10 +1170,8 @@ static int init_state(bpe_cuda_ctx *c, u64 n_local, u64 max_merges, bool encode,
     s.enc_merges = c->d_enc_merges;
     s.enc_total = enc_total;
     s.static_mode = 0;
-    s.use_stream = (u32)c->use_stream;
-    c->want_ranged = c->use_stream && !c->force_census && (u64)c->n_bytes * (u64)c->world >= STATIC_LIMIT;
+    c->want_ranged = (u64)c->n_bytes * (u64)c->world >= STATIC_LIMIT;
     s.want_ranged = (u32)c->want_ranged;
-    // merges may share a pass only on one GPU for now (the all-reduce would grow with the batch) and never in encode
     s.batch_max = (u32)eff_batch(c);
     s.hist_max = (u32)std::max(0, c->smem_hist_max_vocab);
     s.hist_words = 4 * s.hist_max;
@@ -1223,8 +1184,6 @@ static int init_state(bpe_cuda_ctx *c, u64 n_local, u64 max_merges, bool encode,
         s.rcnt[i] = c->d_rcnt[i];
         s.redge[i] = c->d_redge[i];
     }
-    s.pad_ctl = 0u;
-    (void)encode;
     CU(cudaMemcpyAsync(c->d_st, &s, sizeof s, cudaMemcpyHostToDevice, c->stream));
     return 0;
 }
@@ -1265,7 +1224,6 @@ static int run_common(bpe_cuda_ctx *c, u64 max_merges, const bpe_pair_t *enc_mer
     {
         CU(cudaMalloc(&c->d_part, (size_t)c->sel_grid * sizeof(SelPart)));
         CU(cudaMalloc(&c->d_cand, CAND_CAP * sizeof(u32)));
-        CU(cudaMalloc(&c->d_touched, TOUCHED_CAP * sizeof(u32)));
     }
     c->cand_T = 0;
     // fresh table (in the arena the last run left unused, so a big arena stays available for the rehashes)
@@ -1310,7 +1268,7 @@ static int run_common(bpe_cuda_ctx *c, u64 max_merges, const bpe_pair_t *enc_mer
         for (auto &e : c->prof)
             CU(cudaEventCreate(&e));
     }
-    if ((rc = init_state(c, n, max_merges, encode, n_enc)))
+    if ((rc = init_state(c, n, max_merges, n_enc)))
         return rc;
 
     cudaEvent_t ev0, ev1;
@@ -1623,19 +1581,6 @@ static int resolve_pause(bpe_cuda_ctx *c, bool encode)
         repack_kernel<<<RANGE_MAX, 1024, 0, c->stream>>>(c->d_st);
         c->launches++;
     }
-    if (pause & PAUSE_SAME)
-    {
-        // the merge (a == a) is already committed: run its pass with the general kernel
-        resume_kernel<<<1, 1, 0, c->stream>>>(c->d_st);
-        c->launches++;
-        if ((rc = ensure_delta(c, (size_t)(256 + merges_done + 2))))
-            return rc;
-        if ((rc = ensure_xchg(c, (size_t)(256 + merges_done + 2), 0)))
-            return rc;
-        if ((rc = ensure_logs(c, (size_t)(merges_done + 2))))
-            return rc;
-        return enqueue_step(c, (u32)(256 + merges_done - 1), n, encode, false, false);
-    }
     if (pause & PAUSE_STATIC)
     {
         // the select kernel latched static_mode; several GPUs: from here on every rank works on the whole stream;
@@ -1749,23 +1694,6 @@ int bpe_cuda_ctx_create(int device, bpe_cuda_ctx_t **out)
     c->device = device;
     c->debug = getenv("BPE_CUDA_DEBUG") != nullptr;
     c->sm_count = prop.multiProcessorCount;
-    if (const char *e = getenv("BPE_CUDA_INPLACE"))
-        c->inplace = atoi(e);
-    if (const char *e = getenv("BPE_CUDA_L2_PIN"))
-        c->l2_pin = atoi(e);
-    if (c->l2_pin && prop.persistingL2CacheMaxSize > 0)
-    {
-        c->l2_persist_bytes = (size_t)prop.persistingL2CacheMaxSize;
-        c->l2_window_max = (size_t)prop.accessPolicyMaxWindowSize;
-        if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, c->l2_persist_bytes) != cudaSuccess)
-        {
-            cudaGetLastError();
-            c->l2_window_max = 0;
-        }
-        if (c->debug)
-            fprintf(stderr, "[bpe_cuda] L2 %d MB, persisting max %zu MB, window max %zu MB\n", prop.l2CacheSize >> 20,
-                    c->l2_persist_bytes >> 20, c->l2_window_max >> 20);
-    }
     if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess ||
         cudaMalloc(&c->d_st, sizeof(DevState)) != cudaSuccess ||
         cudaMallocHost(&c->h_buf[0], sizeof(DevState)) != cudaSuccess ||
@@ -1795,16 +1723,10 @@ int bpe_cuda_ctx_create(int device, bpe_cuda_ctx_t **out)
             return rc;
         }
     }
-    if (const char *e = getenv("BPE_CUDA_USE_STREAM"))
-        c->use_stream = atoi(e) != 0;
     if (const char *e = getenv("BPE_CUDA_BATCH_MAX"))
         c->batch_max = atoi(e);
     if (const char *e = getenv("BPE_CUDA_RANGES"))
         c->ranges_opt = atoi(e);
-    if (const char *e = getenv("BPE_CUDA_PDL"))
-        c->pdl = atoi(e) != 0;
-    if (const char *e = getenv("BPE_CUDA_SPECULATE"))
-        c->speculate = atoi(e) != 0;
     if (const char *e = getenv("BPE_CUDA_AGRID_MAX"))
         c->agrid_max = std::max(64, atoi(e));
     if (const char *e = getenv("BPE_CUDA_XCHG_TIMEOUT_MS"))
@@ -1861,7 +1783,6 @@ void bpe_cuda_ctx_destroy(bpe_cuda_ctx_t *c)
     table_free(c);
     cudaFree(c->d_part);
     cudaFree(c->d_cand);
-    cudaFree(c->d_touched);
     cudaFree(c->d_merges);
     cudaFree(c->d_nhist);
     cudaFree(c->d_enc_merges);
@@ -2217,22 +2138,12 @@ int bpe_cuda_ctx_set_option(bpe_cuda_ctx_t *c, const char *name, long long value
         c->smem_hist_max_vocab = (int)std::min<long long>(value, 8192);
         return setup_kernels(c);
     }
-    else if (!strcmp(name, "force_census"))
-        c->force_census = (int)value;
     else if (!strcmp(name, "batch_min_z"))
         c->batch_min_z = (int)value;
     else if (!strcmp(name, "batch_max"))
         c->batch_max = (int)value;
     else if (!strcmp(name, "ranges"))
         c->ranges_opt = (int)value;
-    else if (!strcmp(name, "inplace"))
-        c->inplace = (int)(value != 0);
-    else if (!strcmp(name, "pdl"))
-        c->pdl = (int)(value != 0);
-    else if (!strcmp(name, "speculate"))
-        c->speculate = (int)(value != 0);
-    else if (!strcmp(name, "use_stream"))
-        c->use_stream = (int)(value != 0);
     else if (!strcmp(name, "xchg_cap")) // entries per inbox slot at set_comm (test knob: small values force growth)
         c->xcap_opt = (size_t)std::max<long long>(64, value);
     else

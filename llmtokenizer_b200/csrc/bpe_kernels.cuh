@@ -50,7 +50,6 @@ enum : u32
     PAUSE_TIE = 1,    // >= 2 maximal pairs share the winning bucket: chain order decides
     PAUSE_EDGE = 2,   // D sits exactly on a doubling threshold of the merged table
     PAUSE_STATIC = 4, // stream fell below 1,048,576 tokens: reference switches to static slicing
-    PAUSE_SAME = 8,   // (unused since a == b passes run inside replace_stream_kernel; kept for the host's pause handler)
     PAUSE_REBUILD = 16 // the best candidate fell below the list's threshold: the list must be rebuilt
 };
 enum : u32
@@ -114,25 +113,20 @@ struct DevState
     u32 skip; // encode: this rank's pair does not occur anywhere -> no pass
     // loop control
     u32 stop, pause, err, static_mode;
-    u32 use_stream, pad_ctl; // a != b passes run in replace_stream_kernel (bpe_replace.cuh)
     u64 merges_done, max_merges;
     // Stream layout.  DENSE: tok[cur][0..n).  RANGED: the shard is cut into nr ranges that are compacted
     // independently (one CTA each, no prefix scan across CTAs): range c lives at tok[buf][c*rcap ..
     // c*rcap + rcnt[buf][c]); redge[buf][8c..] holds its first three and last two tokens.
     u32 layout, layout_next;
-    u32 want_ranged, pad_wr; // the host runs a != b passes with the streaming kernel: a == b must pause first
+    u32 want_ranged, pad_wr; // the host runs this run's passes above the static limit with replace_stream_kernel
     u32 nr, rmax;
     u64 rcap;
     u32 *rcnt[2];
     u32 *redge[2];
-    u32 rp_done, inplace; // inplace: a RANGED stream is compacted inside its own buffer (tok[0] == tok[1])
+    u32 rp_done, pad_rp;
     u32 rpar[RANGE_MAX];  // a == b passes: per range, epoch << 2 | whole range is one run << 1 | parity of its trailing run
-    u32 *tok_real[2];     // the two allocations; tok[] aliases one of them while RANGED and in place
+    u32 *tok_real[2];     // the two allocations; tok[] aliases one of them while RANGED (tok[0] == tok[1])
     u64 ext_why[8];       // debug statistics: why batch extensions ended (see apply_select_kernel)
-    // delta entries that became non-zero in the current pass (single GPU): apply walks this list instead of
-    // scanning 4 * nb * V mostly-zero counters
-    u32 *touched;
-    u32 ntouched, touched_cap, touched_overflow, use_touched;
     u64 probe_key, probe_slot; // last pair of the stream and its table slot, looked up while the deltas are applied
     u64 dbg[8]; // phase timers of the fused apply+select kernel (ns, summed; BPE_CUDA_DEBUG prints them)
     // pair table: open addressing, key = a | b<<32, meta = murmur3 | count<<32
@@ -1841,8 +1835,6 @@ __device__ __forceinline__ void finish_pass(DevState *st)
         st->layout = st->layout_next;
     }
     st->pending = 0;
-    st->ntouched = 0;
-    st->touched_overflow = 0;
 }
 
 // whole-table mode: K4 alone (select_kernel follows)

@@ -549,7 +549,7 @@ __global__ void __launch_bounds__(V_THREADS, 2) replace_stream_kernel(DevState *
     __shared__ u32 s_ba[BATCH_MAX], s_bb[BATCH_MAX];
     __shared__ __align__(16) u32 s_ab[2 * BATCH_MAX]; // the same pairs interleaved (a0, b0, a1, b1, ...)
 
-    // in and out are the same array when the stream is compacted in place (st->inplace): every tile is
+    // in and out are the same array (the stream is compacted in place, see partition_kernel): every tile is
     // written at or below where it was read, and the storers wait for the next tile's load (whose front
     // halo is the only part of it a store of this tile can reach) before they write
     const u32 *in = st->tok[ibuf] + (u64)cta * rcap;
@@ -1012,8 +1012,8 @@ __global__ void __launch_bounds__(RANGE_MAX) partition_kernel(DevState *st)
         st->nr = nr;
         st->rcap = rcap;
         st->layout = LAYOUT_RANGED;
-        if (st->inplace)
-            st->tok[st->cur ^ 1u] = st->tok[st->cur]; // passes now read and write the same array
+        // passes now read and write the same array (half the working set: late streams stay in L2 from pass to pass)
+        st->tok[st->cur ^ 1u] = st->tok[st->cur];
     }
 }
 

@@ -83,7 +83,7 @@ __device__ __forceinline__ u32 cslot31(u32 doublings_to_come, u64 r)
 }
 
 // ---- begin: new census epoch, geometry, "is it needed at all" ---------------------------------
-__global__ void census_begin_kernel(DevState *st, ResState *rs, int resolver, int force)
+__global__ void census_begin_kernel(DevState *st, ResState *rs, int resolver)
 {
     const bool active = resolver ? (st->stop == STOP_PAUSE) : (st->stop == STOP_RUN);
     if (!active)
@@ -119,7 +119,7 @@ __global__ void census_begin_kernel(DevState *st, ResState *rs, int resolver, in
     }
     if (rs->slices == 1 && !resolver)
         need = 0; // one worker, D keys: handled without a pass (dynamic_regime_census)
-    rs->need = (resolver || force) ? 1u : need;
+    rs->need = resolver ? 1u : need;
 }
 
 // ---- pass 1: first position of every (pair, slice) ---------------------------------------------
