@@ -17,6 +17,9 @@
  *   bpe_cuda_decode           bpe/src/bpe.c:341-394 decompress() with resolve_pair() bpe.c:23-92: ids ->
  *   bpe_cuda_ctx_decode*      bytes through the merge list; byte-exact and NUL-safe (explicit lengths
  *                             instead of the reference's NUL-terminated memo strings)
+ *   bpe_cuda_encode_batch     encode / decode of a batch of independent documents in one call, with
+ *   bpe_cuda_decode_batch     per-document offsets (the ids / bytes of document i are one slice of the
+ *   bpe_cuda_ctx_*_batch      output); additive
  *   bpe_cuda_train_file       bpe/src/bpe.c:130-180 (get_file) + :555 (strlen cut) + :580-584 (widen) in front of the
  *   bpe_cuda_encode_file      path: the file is read in 32 MB pieces through pinned buffers, piece i+1 being read while
  *   bpe_cuda_ctx_upload_file  piece i is copied to the GPU and the pieces before it are widened and counted there
@@ -115,6 +118,19 @@ int bpe_cuda_encode_batch(const uint8_t *bytes, const uint64_t *offsets, size_t 
                           size_t n_merges, uint32_t **tokens_out, uint64_t **tok_offsets_out, size_t *n_tokens,
                           bpe_cuda_stats_t *stats);
 
+/* Inverse of bpe_cuda_encode_batch: document i is tokens[tok_offsets[i] .. tok_offsets[i+1]) (tok_offsets: n_docs + 1
+ * non-decreasing values; tok_offsets[0] need not be 0).  Its bytes are (*bytes_out)[byte_offsets[i] ..
+ * byte_offsets[i+1]) (byte_offsets[0] = 0), identical to bpe_cuda_decode() of its ids alone, so the whole output is
+ * bpe_cuda_decode() of tokens[tok_offsets[0] .. tok_offsets[n_docs]).  Device 0; outputs malloc()'d (*bytes_out with one
+ * terminating 0 after *n_bytes bytes, *byte_offsets_out with n_docs + 1 values).  At most 4,294,967,294 documents.  An
+ * id >= 256 + n_merges fails with BPE_CUDA_ERR_ARG, and bpe_cuda_last_error() names the first document that holds one.
+ * One fixed sequence of four kernel launches whatever the number of documents (none when there is no id).  stats:
+ * n_input = ids, n_tokens = bytes, n_merges, kernel_launches, ms_device (CUDA events around the kernels), ms_h2d,
+ * ms_d2h, ms_total, and table_rehashes = 1 when the call flattened and uploaded the vocabulary. */
+int bpe_cuda_decode_batch(const uint32_t *tokens, const uint64_t *tok_offsets, size_t n_docs, const bpe_pair_t *merges,
+                          size_t n_merges, uint8_t **bytes_out, uint64_t **byte_offsets_out, size_t *n_bytes,
+                          bpe_cuda_stats_t *stats);
+
 void bpe_cuda_free(void *p);
 const char *bpe_cuda_last_error(void);
 int bpe_cuda_device_count(void);
@@ -152,6 +168,16 @@ int bpe_cuda_ctx_encode(bpe_cuda_ctx_t *ctx, const bpe_pair_t *merges, size_t n_
  * stream of batches with one vocabulary pays for it once. */
 int bpe_cuda_ctx_encode_batch(bpe_cuda_ctx_t *ctx, const uint8_t *bytes, const uint64_t *offsets, size_t n_docs,
                               const bpe_pair_t *merges, size_t n_merges, uint32_t *tokens, uint64_t *tok_offsets,
+                              bpe_cuda_stats_t *stats);
+
+/* bpe_cuda_decode_batch() on a context: the n_docs + 1 byte offsets go to the caller's byte_offsets, *n_bytes is the
+ * size of the output, and the bytes stay on the device like those of bpe_cuda_ctx_decode() (fetch them with
+ * bpe_cuda_ctx_decode_download() or bpe_cuda_ctx_device_decoded()).  Leaves the resident shard and the last
+ * train/encode results untouched.  The flattened vocabulary stays on the context and is rebuilt only when the merge list
+ * changes (bpe_cuda_ctx_decode() shares it), so a stream of batches with one vocabulary pays for it once.  After an id
+ * outside the vocabulary (BPE_CUDA_ERR_ARG) the context stays usable. */
+int bpe_cuda_ctx_decode_batch(bpe_cuda_ctx_t *ctx, const uint32_t *tokens, const uint64_t *tok_offsets, size_t n_docs,
+                              const bpe_pair_t *merges, size_t n_merges, uint64_t *byte_offsets, size_t *n_bytes,
                               bpe_cuda_stats_t *stats);
 
 /* Results of the last train/encode on this context. */

@@ -34,6 +34,7 @@ EXPORTS = [
     "bpe_cuda_decode", "bpe_cuda_ctx_decode", "bpe_cuda_ctx_decode_download", "bpe_cuda_ctx_decode_compare",
     "bpe_cuda_ctx_device_decoded", "bpe_cuda_train_file", "bpe_cuda_encode_file", "bpe_cuda_ctx_upload_file",
     "bpe_cuda_ctx_truncate", "bpe_cuda_ctx_download_pageable", "bpe_cuda_encode_batch", "bpe_cuda_ctx_encode_batch",
+    "bpe_cuda_decode_batch", "bpe_cuda_ctx_decode_batch",
 ]
 
 _lib = None
@@ -72,6 +73,12 @@ def load():
     lib.bpe_cuda_ctx_encode_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t,
                                               C.c_void_p, C.c_void_p, P(Stats)]
     lib.bpe_cuda_ctx_encode_batch.restype = C.c_int
+    lib.bpe_cuda_decode_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, P(P(C.c_uint8)),
+                                          P(P(C.c_uint64)), P(C.c_size_t), P(Stats)]
+    lib.bpe_cuda_decode_batch.restype = C.c_int
+    lib.bpe_cuda_ctx_decode_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t,
+                                              C.c_void_p, P(C.c_size_t), P(Stats)]
+    lib.bpe_cuda_ctx_decode_batch.restype = C.c_int
     lib.bpe_cuda_free.argtypes = [C.c_void_p]
     lib.bpe_cuda_free.restype = None
     lib.bpe_cuda_last_error.restype = C.c_char_p

@@ -159,6 +159,47 @@ def encode_batch(docs, merges):
     return t, o, st.as_dict()
 
 
+def _as_id_batch(docs):
+    """docs: a sequence of id arrays, or a (uint32 ids, uint64 offsets) tuple as encode_batch() returns ->
+    (ids, offsets) arrays.  As in _as_batch, only an offsets array of dtype uint64 selects the tuple form."""
+    if (isinstance(docs, tuple) and len(docs) == 2 and isinstance(docs[0], np.ndarray) and isinstance(docs[1], np.ndarray)
+            and docs[1].dtype == np.uint64):
+        ids = np.ascontiguousarray(np.asarray(docs[0], dtype=np.uint32).reshape(-1))
+        off = np.ascontiguousarray(docs[1])
+        if off.ndim != 1 or off.size < 1 or int(off[-1]) > ids.size:
+            raise ValueError("offsets must be 1-D, hold n_docs + 1 values and end inside the id array")
+        return ids, off
+    parts = [np.asarray(d, dtype=np.uint32).reshape(-1) for d in docs]
+    off = np.zeros(len(parts) + 1, dtype=np.uint64)
+    np.cumsum([p.size for p in parts], out=off[1:])
+    ids = np.concatenate(parts) if parts else np.zeros(0, dtype=np.uint32)
+    return np.ascontiguousarray(ids, dtype=np.uint32), off
+
+
+def decode_batch(docs, merges):
+    """Decode every id sequence of a batch in one call on device 0 -> (bytes, offsets uint64[n_docs + 1], stats):
+    bytes[offsets[i]:offsets[i+1]] == decode(docs[i], merges)[0].  decode_batch(encode_batch(d, m)[:2], m) round-trips."""
+    lib = _lib.load()
+    ids, off = _as_id_batch(docs)
+    mg = np.ascontiguousarray(np.asarray(merges, dtype=np.uint32).reshape(-1, 2))
+    out = C.POINTER(C.c_uint8)()
+    boff = C.POINTER(C.c_uint64)()
+    nb = C.c_size_t()
+    st = Stats()
+    rc = lib.bpe_cuda_decode_batch(ids.ctypes.data if ids.size else None, off.ctypes.data, off.size - 1,
+                                   mg.ctypes.data if mg.size else None, mg.shape[0], C.byref(out), C.byref(boff),
+                                   C.byref(nb), C.byref(st))
+    if rc:
+        raise BpeCudaError(rc)
+    try:
+        b = C.string_at(out, nb.value)
+        o = np.ctypeslib.as_array(boff, shape=(off.size,)).copy()
+    finally:
+        lib.bpe_cuda_free(out)
+        lib.bpe_cuda_free(boff)
+    return b, o, st.as_dict()
+
+
 def decode(tokens, merges):
     """ids -> bytes through the merge list (what decompress() computes, bpe.c:341-394) -> (bytes, stats)."""
     lib = _lib.load()
@@ -268,6 +309,28 @@ class Context:
         if rc:
             raise BpeCudaError(rc)
         return buf.tobytes()
+
+    def decode_batch(self, docs, merges, download=True):
+        """decode_batch() on this context -> (bytes, offsets, stats).  With download=False the bytes stay on the device
+        (as after decode()) and the first element is their count.  The resident shard and the last train/encode
+        results stay as they are, and the flattened vocabulary is kept for the next call with the same merge list."""
+        ids, off = _as_id_batch(docs)
+        mg = np.ascontiguousarray(np.asarray(merges, dtype=np.uint32).reshape(-1, 2))
+        boff = np.empty(off.size, dtype=np.uint64)
+        nb = C.c_size_t()
+        st = Stats()
+        rc = self.lib.bpe_cuda_ctx_decode_batch(self.h, ids.ctypes.data if ids.size else None, off.ctypes.data, off.size - 1,
+                                                mg.ctypes.data if mg.size else None, mg.shape[0], boff.ctypes.data,
+                                                C.byref(nb), C.byref(st))
+        if rc:
+            raise BpeCudaError(rc)
+        if not download:
+            return nb.value, boff, st.as_dict()
+        buf = np.zeros(nb.value, dtype=np.uint8)
+        rc = self.lib.bpe_cuda_ctx_decode_download(self.h, buf.ctypes.data if nb.value else None)
+        if rc:
+            raise BpeCudaError(rc)
+        return buf.tobytes(), boff, st.as_dict()
 
     def decode_mismatches(self):
         """Bytes of the last decode that differ from the resident shard (compared on the device)."""

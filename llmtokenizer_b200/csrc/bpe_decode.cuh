@@ -11,6 +11,8 @@
 //                            shared memory, written out as aligned 16-byte vectors
 // HBM traffic per id: 4 B read twice (D1, D3) + its expansion written once; the blob (a few hundred
 // KB) stays in L1/L2.  Byte-exact and NUL-safe (lengths are explicit), unlike the char* original.
+// A batch of documents (D4) runs decode_batch_tiles_kernel, D1, D2 and decode_expand_kernel<true>, which also writes
+// the byte offset of every document: O(1) per document and per tile on top of the plain decode.
 #pragma once
 #include "bpe_kernels.cuh"
 
@@ -116,11 +118,49 @@ __global__ void __launch_bounds__(1024) decode_scan_kernel(u64 *tile_sum, u64 nt
         tile_sum[nt] = s_carry;
 }
 
+// D4 (batch decode): the documents of a batch, for decode_expand_kernel<true>.  Entry i of tok_off (i <= n_docs, the
+// last one being the batch's end) starts at id tok_off[i] - base; the ones that start inside tile t are
+// tile_doc[t] .. tile_doc[t+1]-1, and the last tile also takes those that start at the end of the batch.
+struct DecodeDocs
+{
+    const u64 *tok_off; // [n_docs + 1]
+    u64 base;           // tok_off[0]
+    u32 *tile_doc;       // [tiles + 1], written by decode_batch_tiles_kernel
+    u64 *byte_off;       // [n_docs + 1] out
+};
+
+// D4 helper: tile_doc[t] = first entry of tok_off that starts at or after tile t (one binary search per tile);
+// tile_doc[nt] = n_docs + 1.
+__global__ void __launch_bounds__(256) decode_batch_tiles_kernel(const u64 *__restrict__ tok_off, u32 n_ends, u64 base,
+                                                                 u64 nt, u32 *__restrict__ tile_doc)
+{
+    const u64 t = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t > nt)
+        return;
+    u32 lo = t < nt ? 0 : n_ends, hi = n_ends;
+    if (t < nt)
+    {
+        const u64 start = base + t * DEC_TILE;
+        while (lo < hi)
+        {
+            const u32 mid = lo + (hi - lo) / 2;
+            if (tok_off[mid] < start)
+                lo = mid + 1;
+            else
+                hi = mid;
+        }
+    }
+    tile_doc[t] = lo;
+}
+
 // D3: expand the ids of one tile.  Thread t owns DEC_PER_THREAD CONSECUTIVE ids so that its bytes are
-// one contiguous run.
+// one contiguous run.  The body stays in the kernel (not an inlined helper) so that <false> compiles to the same code
+// as before D4 existed.  With DOCS (D4), also the byte offset of every document that starts in the tile: the thread
+// that owns its first id knows where that thread's bytes start (s_pos), plus at most DEC_PER_THREAD - 1 lengths.
+template <bool DOCS>
 __global__ void __launch_bounds__(DEC_THREADS) decode_expand_kernel(const u32 *__restrict__ tok, u64 n, DecodeVocab v,
                                                                     const u64 *__restrict__ tile_off,
-                                                                    uint8_t *__restrict__ out)
+                                                                    uint8_t *__restrict__ out, DecodeDocs d)
 {
     __shared__ u64 s_warp[DEC_THREADS / 32];
     __shared__ __align__(16) uint8_t s_stage[DEC_STAGE_BYTES + 16];
@@ -152,6 +192,28 @@ __global__ void __launch_bounds__(DEC_THREADS) decode_expand_kernel(const u32 *_
     u64 pos = before + incl - mine; // offset inside the tile's output
     const u64 o0 = tile_off[blockIdx.x];
     const u64 tile_bytes = tile_off[blockIdx.x + 1] - o0;
+    if constexpr (DOCS)
+    {
+        __shared__ u64 s_pos[DEC_THREADS];
+        s_pos[threadIdx.x] = pos;
+        __syncthreads();
+        const u64 lo = (u64)blockIdx.x * DEC_TILE;
+        const u64 tile_ids = n - lo < (u64)DEC_TILE ? n - lo : (u64)DEC_TILE;
+        const u64 end = d.tile_doc[blockIdx.x + 1];
+        for (u64 i = d.tile_doc[blockIdx.x] + threadIdx.x; i < end; i += DEC_THREADS)
+        {
+            const u64 j = d.tok_off[i] - d.base - lo; // first id of document i, inside the tile
+            u64 b = tile_bytes;                       // (j == tile_ids: it starts at the end of the batch)
+            if (j < tile_ids)
+            {
+                const u32 th = (u32)(j / DEC_PER_THREAD);
+                b = s_pos[th];
+                for (u64 k = lo + (u64)th * DEC_PER_THREAD; k < lo + j; k++)
+                    b += v.len[tok[k]];
+            }
+            d.byte_off[i] = o0 + b;
+        }
+    }
     if (tile_bytes <= DEC_STAGE_BYTES)
     {
         // stage with the same 16-byte phase as the destination, then store whole vectors

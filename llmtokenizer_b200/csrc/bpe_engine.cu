@@ -194,6 +194,12 @@ struct bpe_cuda_ctx
     uint8_t *d_dec_blob = nullptr, *d_dec_out = nullptr;
     u64 *d_dec_tiles = nullptr;
     size_t dec_vocab_cap = 0, dec_blob_cap = 0, dec_out_cap = 0, dec_tiles_cap = 0, dec_n_out = 0;
+    bool dec_valid = false;                 // the vocabulary on the device is the flattening of dec_merges
+    std::vector<bpe_pair_t> dec_merges;
+    // batch decode: the batch's ids and token offsets, first document per tile, byte offsets
+    u32 *d_dbtok = nullptr, *d_dbtile = nullptr;
+    u64 *d_dbtoff = nullptr, *d_dbboff = nullptr;
+    size_t dbtok_cap = 0, dbtile_cap = 0, dbtoff_cap = 0, dbboff_cap = 0;
     u32 *d_rank = nullptr;
     size_t first_cap = 0; // entries (slots * slices)
     u32 *d_pos_slot = nullptr;
@@ -1800,7 +1806,8 @@ void bpe_cuda_ctx_destroy(bpe_cuda_ctx_t *c)
     cudaFree(c->d_tile_off);
     for (void *p : {(void *)c->d_bb, (void *)c->d_btok, (void *)c->d_brk, (void *)c->d_bdoc, (void *)c->d_btoff,
                     (void *)c->d_blen, (void *)c->d_border, (void *)c->d_bseg, (void *)c->d_bsegs, (void *)c->d_rt_key, (void *)c->d_rt_rank,
-                    (void *)c->d_bnext, (void *)c->d_bmerges})
+                    (void *)c->d_bnext, (void *)c->d_bmerges, (void *)c->d_dbtok, (void *)c->d_dbtile, (void *)c->d_dbtoff,
+                    (void *)c->d_dbboff})
         cudaFree(p);
     if (c->stream)
         cudaStreamDestroy(c->stream);
@@ -2213,36 +2220,79 @@ template <class T> static int dec_reserve(T *&p, size_t &cap, size_t need)
 }
 }
 
-// Expand d_tok[0..n) (device) into c->d_dec_out; *n_bytes = size of the expansion.
-static int decode_device(bpe_cuda_ctx *c, const u32 *d_tok, u64 n, const bpe_pair_t *merges, size_t n_merges, size_t *n_bytes)
+// The flattened vocabulary of the merge list on the device (d_dec_len, d_dec_off, d_dec_blob).  It is rebuilt only
+// when the list differs from the one it was built from, so a stream of decodes with one vocabulary flattens and
+// uploads it once.  *rebuilt says whether this call did.
+static int dec_vocab(bpe_cuda_ctx *c, const bpe_pair_t *merges, size_t n_merges, bool *rebuilt)
 {
+    *rebuilt = false;
+    if (c->dec_valid && c->dec_merges.size() == n_merges &&
+        (!n_merges || !memcmp(c->dec_merges.data(), merges, n_merges * sizeof(bpe_pair_t))))
+        return 0;
     int rc;
-    CU(cudaSetDevice(c->device));
+    c->dec_valid = false; // until the upload has completed
     std::vector<u32> len, off;
     std::vector<uint8_t> blob;
     if ((rc = decode_flatten(merges, n_merges, len, off, blob)))
         return rc;
     const size_t V = len.size();
-    const u64 nt = (n + DEC_TILE - 1) / DEC_TILE;
     size_t cap2 = c->dec_vocab_cap;
     if ((rc = dec_reserve(c->d_dec_len, c->dec_vocab_cap, V)) || (rc = dec_reserve(c->d_dec_off, cap2, V)) ||
-        (rc = dec_reserve(c->d_dec_blob, c->dec_blob_cap, blob.size())) ||
-        (rc = dec_reserve(c->d_dec_tiles, c->dec_tiles_cap, nt + 2)))
+        (rc = dec_reserve(c->d_dec_blob, c->dec_blob_cap, blob.size())))
         return rc;
     CU(cudaMemcpyAsync(c->d_dec_len, len.data(), V * sizeof(u32), cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(c->d_dec_off, off.data(), V * sizeof(u32), cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(c->d_dec_blob, blob.data(), blob.size(), cudaMemcpyHostToDevice, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    c->dec_merges.assign(merges, merges + n_merges);
+    c->dec_valid = true;
+    *rebuilt = true;
+    return 0;
+}
+
+// Expand d_tok[0..n) (device) into c->d_dec_out through the vocabulary dec_vocab() left on the device; *n_bytes = size
+// of the expansion, *ms = device time of the kernels (CUDA events, without the host round trip between D2 and D3).
+// With docs (batch decode, n > 0), also the byte offset of each of its n_ends entries.  An id outside the vocabulary
+// returns BPE_CUDA_ERR_ARG before anything is expanded.
+static int decode_run(bpe_cuda_ctx *c, const u32 *d_tok, u64 n, const DecodeDocs *docs, u64 n_ends, size_t *n_bytes, float *ms)
+{
+    int rc;
+    const size_t V = 256 + c->dec_merges.size();
+    const u64 nt = (n + DEC_TILE - 1) / DEC_TILE;
+    if ((rc = dec_reserve(c->d_dec_tiles, c->dec_tiles_cap, nt + 2)))
+        return rc;
+    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+    struct EvGuard
+    {
+        cudaEvent_t *e;
+        ~EvGuard()
+        {
+            for (int k = 0; k < 4; k++)
+                if (e[k])
+                    cudaEventDestroy(e[k]);
+        }
+    } ev_guard{ev};
+    for (int k = 0; k < 4; k++)
+        CU(cudaEventCreate(&ev[k]));
     u64 *d_total = c->d_dec_tiles + nt;     // written by the scan
     u32 *d_err = reinterpret_cast<u32 *>(c->d_dec_tiles + nt + 1);
     CU(cudaMemsetAsync(c->d_dec_tiles + nt, 0, 2 * sizeof(u64), c->stream));
     DecodeVocab v{c->d_dec_len, c->d_dec_off, c->d_dec_blob, (u32)V};
     c->dec_n_out = 0;
+    CU(cudaEventRecord(ev[0], c->stream));
     if (n)
     {
+        if (docs)
+        {
+            decode_batch_tiles_kernel<<<(unsigned)((nt + 1 + 255) / 256), 256, 0, c->stream>>>(docs->tok_off, (u32)n_ends,
+                                                                                               docs->base, nt, docs->tile_doc);
+            c->launches++;
+        }
         decode_len_kernel<<<(unsigned)nt, DEC_THREADS, 0, c->stream>>>(d_tok, n, v, c->d_dec_tiles, d_err);
         decode_scan_kernel<<<1, 1024, 0, c->stream>>>(c->d_dec_tiles, nt);
         c->launches += 2;
     }
+    CU(cudaEventRecord(ev[1], c->stream));
     u64 h[2] = {0, 0};
     CU(cudaMemcpyAsync(h, d_total, sizeof h, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
@@ -2253,16 +2303,46 @@ static int decode_device(bpe_cuda_ctx *c, const u32 *d_tok, u64 n, const bpe_pai
     }
     if ((rc = dec_reserve(c->d_dec_out, c->dec_out_cap, (size_t)h[0] + 16)))
         return rc;
+    CU(cudaEventRecord(ev[2], c->stream));
     if (n)
     {
-        decode_expand_kernel<<<(unsigned)nt, DEC_THREADS, 0, c->stream>>>(d_tok, n, v, c->d_dec_tiles, c->d_dec_out);
+        if (docs)
+            decode_expand_kernel<true><<<(unsigned)nt, DEC_THREADS, 0, c->stream>>>(d_tok, n, v, c->d_dec_tiles, c->d_dec_out,
+                                                                                  *docs);
+        else
+            decode_expand_kernel<false><<<(unsigned)nt, DEC_THREADS, 0, c->stream>>>(d_tok, n, v, c->d_dec_tiles, c->d_dec_out,
+                                                                                   DecodeDocs{});
         c->launches++;
     }
     CU(cudaGetLastError());
+    CU(cudaEventRecord(ev[3], c->stream));
     CU(cudaStreamSynchronize(c->stream));
+    float m01 = 0, m23 = 0;
+    CU(cudaEventElapsedTime(&m01, ev[0], ev[1]));
+    CU(cudaEventElapsedTime(&m23, ev[2], ev[3]));
+    *ms = m01 + m23;
     c->dec_n_out = (size_t)h[0];
+    *n_bytes = (size_t)h[0];
+    return 0;
+}
+
+// Expand d_tok[0..n) (device) into c->d_dec_out; *n_bytes = size of the expansion, *ms = its device time.
+static int decode_device(bpe_cuda_ctx *c, const u32 *d_tok, u64 n, const bpe_pair_t *merges, size_t n_merges, size_t *n_bytes,
+                         float *ms = nullptr)
+{
+    int rc;
+    CU(cudaSetDevice(c->device));
+    bool rebuilt;
+    if ((rc = dec_vocab(c, merges, n_merges, &rebuilt)))
+        return rc;
+    size_t nb = 0;
+    float t = 0;
+    if ((rc = decode_run(c, d_tok, n, nullptr, 0, &nb, &t)))
+        return rc;
     if (n_bytes)
-        *n_bytes = (size_t)h[0];
+        *n_bytes = nb;
+    if (ms)
+        *ms = t;
     return 0;
 }
 
@@ -2331,13 +2411,14 @@ int bpe_cuda_decode(const uint32_t *tokens, size_t n_tokens, const bpe_pair_t *m
     u32 *d_tok = nullptr;
     uint8_t *out = nullptr;
     size_t nb = 0;
+    float ms = 0;
     auto body = [&]() -> int {
         if (n_tokens)
         {
             CU(cudaMalloc(&d_tok, n_tokens * sizeof(u32)));
             CU(cudaMemcpyAsync(d_tok, tokens, n_tokens * sizeof(u32), cudaMemcpyHostToDevice, c->stream));
         }
-        int r = decode_device(c, d_tok, n_tokens, merges, n_merges, &nb);
+        int r = decode_device(c, d_tok, n_tokens, merges, n_merges, &nb, &ms);
         if (r)
             return r;
         out = (uint8_t *)malloc(nb + 1); // +1: room for the terminator decompress() appends (bpe.c:390)
@@ -2359,6 +2440,7 @@ int bpe_cuda_decode(const uint32_t *tokens, size_t n_tokens, const bpe_pair_t *m
         stats->n_merges = n_merges;
         stats->n_tokens = nb;
         stats->kernel_launches = c->launches;
+        stats->ms_device = ms;
         stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     }
     bpe_cuda_ctx_destroy(c);
@@ -2373,6 +2455,17 @@ int bpe_cuda_decode(const uint32_t *tokens, size_t n_tokens, const bpe_pair_t *m
 }
 
 // ---- batch encode (bpe_encode_batch.cuh) ------------------------------------------------------
+static int check_merges(const bpe_pair_t *merges, size_t n_merges)
+{
+    for (size_t r = 0; r < n_merges; r++)
+        if (merges[r].a >= 256 + r || merges[r].b >= 256 + r)
+        {
+            set_error("merge %zu refers to an id that does not exist yet", r);
+            return BPE_CUDA_ERR_ARG;
+        }
+    return 0;
+}
+
 // Every argument is checked before any device call, so that a bad call fails the same way with or without a GPU.
 static int batch_check(const uint8_t *bytes, const uint64_t *offsets, size_t n_docs, const bpe_pair_t *merges,
                        size_t n_merges)
@@ -2405,13 +2498,7 @@ static int batch_check(const uint8_t *bytes, const uint64_t *offsets, size_t n_d
         set_error("invalid argument: NULL bytes");
         return BPE_CUDA_ERR_ARG;
     }
-    for (size_t r = 0; r < n_merges; r++)
-        if (merges[r].a >= 256 + r || merges[r].b >= 256 + r)
-        {
-            set_error("merge %zu refers to an id that does not exist yet", r);
-            return BPE_CUDA_ERR_ARG;
-        }
-    return 0;
+    return check_merges(merges, n_merges);
 }
 
 // Encode the batch on the device.  On success the ids are c->d_brk[0 .. *n_tokens) and the offsets c->d_btoff[0 ..
@@ -2685,6 +2772,190 @@ int bpe_cuda_encode_batch(const uint8_t *bytes, const uint64_t *offsets, size_t 
     *tokens_out = tok;
     *tok_offsets_out = toff;
     *n_tokens = m;
+    return 0;
+}
+
+// ---- batch decode (D4 in bpe_decode.cuh) ------------------------------------------------------
+// Every argument is checked before any device call, as batch_check() does for encode.
+static int decode_batch_check(const uint32_t *tokens, const uint64_t *tok_offsets, size_t n_docs, const bpe_pair_t *merges,
+                              size_t n_merges)
+{
+    if (!tok_offsets || (!merges && n_merges))
+    {
+        set_error("invalid argument: NULL tok_offsets or merges");
+        return BPE_CUDA_ERR_ARG;
+    }
+    if (n_docs >= 0xFFFFFFFFu) // n_docs + 1 entries are indexed with 32 bits on the device
+    {
+        set_error("invalid argument: %zu documents (at most 4,294,967,294 in one batch)", n_docs);
+        return BPE_CUDA_ERR_ARG;
+    }
+    for (size_t i = 0; i < n_docs; i++)
+        if (tok_offsets[i + 1] < tok_offsets[i])
+        {
+            set_error("invalid argument: tok_offsets[%zu] < tok_offsets[%zu] (offsets must not decrease)", i + 1, i);
+            return BPE_CUDA_ERR_ARG;
+        }
+    if (!tokens && tok_offsets[n_docs] > tok_offsets[0])
+    {
+        set_error("invalid argument: NULL tokens");
+        return BPE_CUDA_ERR_ARG;
+    }
+    return check_merges(merges, n_merges);
+}
+
+// Decode the batch on the device: the bytes go to c->d_dec_out[0 .. *n_bytes), the byte offsets to the host array
+// byte_offsets[0 .. n_docs].  st gets every field of the result but ms_total; its ms_d2h covers the offsets.
+static int decode_batch_run(bpe_cuda_ctx *c, const uint32_t *tokens, const uint64_t *tok_offsets, size_t n_docs,
+                            const bpe_pair_t *merges, size_t n_merges, uint64_t *byte_offsets, size_t *n_bytes,
+                            bpe_cuda_stats_t *st)
+{
+    int rc;
+    CU(cudaSetDevice(c->device));
+    memset(st, 0, sizeof *st);
+    const u64 base = tok_offsets[0], N = tok_offsets[n_docs] - base;
+    st->n_input = N;
+    st->n_merges = n_merges;
+    c->dec_n_out = 0;
+    *n_bytes = 0;
+    if (!N) // no id at all: every document is empty, and nothing is launched
+    {
+        memset(byte_offsets, 0, (n_docs + 1) * sizeof(uint64_t));
+        return 0;
+    }
+    const u64 nt = (N + DEC_TILE - 1) / DEC_TILE;
+    bool rebuilt = false;
+    {
+        const auto h0 = std::chrono::steady_clock::now();
+        if ((rc = dec_vocab(c, merges, n_merges, &rebuilt)) || (rc = dec_reserve(c->d_dbtok, c->dbtok_cap, (size_t)N)) ||
+            (rc = dec_reserve(c->d_dbtoff, c->dbtoff_cap, n_docs + 1)) ||
+            (rc = dec_reserve(c->d_dbboff, c->dbboff_cap, n_docs + 1)) || (rc = dec_reserve(c->d_dbtile, c->dbtile_cap, nt + 1)))
+            return rc;
+        CU(cudaMemcpyAsync(c->d_dbtok, tokens + base, N * sizeof(u32), cudaMemcpyHostToDevice, c->stream));
+        CU(cudaMemcpyAsync(c->d_dbtoff, tok_offsets, (n_docs + 1) * sizeof(u64), cudaMemcpyHostToDevice, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+        st->ms_h2d = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - h0).count();
+    }
+    const DecodeDocs d{c->d_dbtoff, base, c->d_dbtile, c->d_dbboff};
+    const u64 l0 = c->launches;
+    size_t nb = 0;
+    float ms = 0;
+    rc = decode_run(c, c->d_dbtok, N, &d, n_docs + 1, &nb, &ms);
+    if (rc == BPE_CUDA_ERR_ARG)
+    {
+        // the device only says that some id is outside the vocabulary; the host still holds the ids
+        const size_t V = 256 + n_merges;
+        const uint32_t *t = tokens + base;
+        u64 k = 0;
+        while (k < N && t[k] < V)
+            k++;
+        if (k < N)
+        {
+            const size_t doc = (size_t)(std::upper_bound(tok_offsets, tok_offsets + n_docs + 1, base + k) - tok_offsets) - 1;
+            set_error("decode_batch: document %zu holds id %u, outside the vocabulary (%zu entries)", doc, t[k], V);
+        }
+    }
+    if (rc)
+        return rc;
+    const auto h0 = std::chrono::steady_clock::now();
+    CU(cudaMemcpyAsync(byte_offsets, c->d_dbboff, (n_docs + 1) * sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    st->ms_d2h = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - h0).count();
+    st->n_tokens = nb;
+    st->kernel_launches = c->launches - l0;
+    st->table_rehashes = rebuilt;
+    st->ms_device = ms;
+    *n_bytes = nb;
+    return 0;
+}
+
+int bpe_cuda_ctx_decode_batch(bpe_cuda_ctx_t *c, const uint32_t *tokens, const uint64_t *tok_offsets, size_t n_docs,
+                              const bpe_pair_t *merges, size_t n_merges, uint64_t *byte_offsets, size_t *n_bytes,
+                              bpe_cuda_stats_t *stats)
+{
+    int rc = decode_batch_check(tokens, tok_offsets, n_docs, merges, n_merges);
+    if (rc)
+        return rc;
+    if (!byte_offsets || !n_bytes)
+    {
+        set_error("invalid argument: NULL output buffer");
+        return BPE_CUDA_ERR_ARG;
+    }
+    if (!c)
+    {
+        set_error("invalid argument: NULL context");
+        return BPE_CUDA_ERR_ARG;
+    }
+    const auto t0 = std::chrono::steady_clock::now();
+    bpe_cuda_stats_t st;
+    if ((rc = decode_batch_run(c, tokens, tok_offsets, n_docs, merges, n_merges, byte_offsets, n_bytes, &st)))
+        return rc;
+    st.ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats)
+        *stats = st;
+    return 0;
+}
+
+int bpe_cuda_decode_batch(const uint32_t *tokens, const uint64_t *tok_offsets, size_t n_docs, const bpe_pair_t *merges,
+                          size_t n_merges, uint8_t **bytes_out, uint64_t **byte_offsets_out, size_t *n_bytes,
+                          bpe_cuda_stats_t *stats)
+{
+    if (!bytes_out || !byte_offsets_out || !n_bytes)
+    {
+        set_error("invalid argument: NULL output pointer");
+        return BPE_CUDA_ERR_ARG;
+    }
+    *bytes_out = nullptr;
+    *byte_offsets_out = nullptr;
+    *n_bytes = 0;
+    int rc = decode_batch_check(tokens, tok_offsets, n_docs, merges, n_merges);
+    if (rc)
+        return rc;
+    const auto t0 = std::chrono::steady_clock::now();
+    bpe_cuda_ctx_t *c = nullptr;
+    if ((rc = bpe_cuda_ctx_create(0, &c)))
+        return rc;
+    bpe_cuda_stats_t st;
+    size_t nb = 0;
+    uint8_t *out = nullptr;
+    uint64_t *boff = nullptr;
+    auto body = [&]() -> int {
+        boff = (uint64_t *)malloc((n_docs + 1) * sizeof(uint64_t));
+        if (!boff)
+        {
+            set_error("out of host memory");
+            return BPE_CUDA_ERR_NOMEM;
+        }
+        int r = decode_batch_run(c, tokens, tok_offsets, n_docs, merges, n_merges, boff, &nb, &st);
+        if (r)
+            return r;
+        out = (uint8_t *)malloc(nb + 1); // +1: the terminator bpe_cuda_decode() appends too
+        if (!out)
+        {
+            set_error("out of host memory");
+            return BPE_CUDA_ERR_NOMEM;
+        }
+        out[nb] = 0;
+        const auto h0 = std::chrono::steady_clock::now();
+        if ((r = bpe_cuda_ctx_decode_download(c, out)))
+            return r;
+        st.ms_d2h += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - h0).count();
+        return 0;
+    };
+    rc = body();
+    bpe_cuda_ctx_destroy(c);
+    if (rc)
+    {
+        free(out);
+        free(boff);
+        return rc;
+    }
+    st.ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats)
+        *stats = st;
+    *bytes_out = out;
+    *byte_offsets_out = boff;
+    *n_bytes = nb;
     return 0;
 }
 
