@@ -60,6 +60,14 @@ def _tie_heavy(copies=60):
     return np.concatenate(parts)
 
 
+def _wide_ties(n=88_000):
+    # n random bytes from 1..255, twice: nearly every pair count is 2, so every iteration is a hash-table tie-break.
+    # Trained to exhaustion each copy collapses to one token after about 70,300 merges, so ids past 65,535 are born
+    # in the static regime (the stream never holds more than 2 n tokens)
+    r = np.random.default_rng(65536).integers(1, 256, n, dtype=np.uint8)
+    return np.concatenate([r, r])
+
+
 # key -> (input factory, merge cap [0 = to exhaustion])
 TRAIN_CASES = {
     "zipfa6m_300": (lambda: corpus(0, 6_000_000, 99), 300),
@@ -83,6 +91,8 @@ TRAIN_CASES = {
     "ties1m2_exh": (_tie_heavy, 0),
     # 4.3 M tokens that stay above the static limit for all 1,000 merges, 4 of them same-bucket ties
     "ties4m_1000": (lambda: _tie_heavy(220), 1000),
+    # ids past 65,535 (70,306 merges, 3,599 same-bucket ties), all born in the static regime
+    "wideties88k_exh": (_wide_ties, 0),
 }
 for _r in (1, 5, 64, 0):
     for _i in range(3):

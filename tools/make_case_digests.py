@@ -26,6 +26,8 @@ def one(key):
     else:
         d = pc.compute_encode(o, key)
         info = f"{d['n_ids']} ids"
+    d["made_by"] = f"tools/make_case_digests.py {key} (oracle FAST_CF mode, 1 thread)"
+    d["oracle_seconds"] = round(time.time() - t0, 1)
     pc.save(key, d)
     return key, time.time() - t0, info
 

@@ -5,6 +5,7 @@ the 1 GB corpus.
 
   python tools/make_full_golden.py c1_exhaustion                       # random_text.txt to exhaustion (config 1)
   python tools/make_full_golden.py c3_full 1000000000 4321 32000 1     # name, bytes, seed, merges, kind (1 = zipf_bytes)
+  python tools/make_full_golden.py c5_chunk0_70k 125000000 8888 70000 1   # ids past 65,535 (22 minutes, 8 threads)
 
 BO_WORKERS=n (default: all cores) splits the oracle's two whole-array loops over helper threads (same results,
 tests/test_oracle.py); the 1 GB corpus then takes about an hour instead of most of a day.
@@ -55,7 +56,8 @@ def main():
            "ids_sha256": sha(ids), "same_bucket_ties": int(st["same_bucket_ties"]),
            "threshold_edges": int(st["threshold_edges"]), "final_distinct": int(st["final_distinct"]),
            "thread_buckets": [int(x) for x in st["thread_buckets"]],
-           "made_by": f"tools/make_full_golden.py (oracle FAST_CF mode, {workers} helper threads)", "oracle_seconds": round(time.time() - t0, 1)}
+           "made_by": f"tools/make_full_golden.py {' '.join(sys.argv[1:])} (oracle FAST_CF mode, {workers} helper threads)",
+           "oracle_seconds": round(time.time() - t0, 1)}
     np.savez_compressed(os.path.join(ROOT, "tests", "golden", "full", name + "_merges.npz"), merges=m.astype(np.uint32))
     with open(os.path.join(ROOT, "tests", "golden", name + ".json"), "w") as f:
         json.dump(out, f, indent=1)
