@@ -74,6 +74,7 @@ typedef struct
     uint64_t replace_passes;   /* passes over the stream (a pass may carry several merges)            */
     uint64_t batch_merges;     /* merges that rode along in another merge's pass                       */
     uint64_t batch_passes;     /* passes that carried more than one merge                              */
+    uint64_t sparse_passes;    /* passes that ran on the sparse (byte-anchored, occurrence-indexed) layout */
 } bpe_cuda_stats_t;
 
 #define BPE_CUDA_OK 0

@@ -9,6 +9,7 @@
 #include "../../include/bpe_cuda.h"
 #include "bpe_kernels.cuh"
 #include "bpe_replace.cuh"
+#include "bpe_sparse.cuh"
 #include "bpe_resolver.cuh"
 #include "bpe_decode.cuh"
 #include "bpe_encode_batch.cuh"
@@ -254,6 +255,13 @@ struct bpe_cuda_ctx
     std::vector<cudaEvent_t> prof;
     std::vector<unsigned char> prof_tag;
     size_t prof_used = 0;
+    // LAYOUT_SPARSE (bpe_sparse.cuh): frozen pair index, creation lists, byte length per id, scan scratch
+    u64 *d_ikey = nullptr;
+    u32 *d_ioff = nullptr, *d_icur = nullptr, *d_ipos = nullptr, *d_pool = nullptr, *d_sp_tsum = nullptr;
+    u64 *d_pass_buf = nullptr;
+    size_t ikey_cap = 0, icur_cap = 0, ioff_cap = 0, ipos_cap = 0, pool_cap = 0, pass_cap = 0, sp_tsum_cap = 0;
+    u32 *d_slen = nullptr, *d_cl_off = nullptr, *d_cl_cnt = nullptr;
+    size_t sp_vcap = 0;
     // results
     size_t res_n_merges = 0, res_n_tokens = 0;
     bpe_cuda_stats_t stats;
@@ -804,7 +812,7 @@ static int enqueue_select(bpe_cuda_ctx *c, bool encode)
 
 // One merge step for the committed merge that creates id z: [census] -> replace (+scan+deltas) ->
 // [edge record, ncclAllReduce] -> apply deltas + select the next merge.
-static int enqueue_step(bpe_cuda_ctx *c, u32 z, u64 n_upper, bool encode, bool census, bool ranged, u64 z_ub = 0)
+static int enqueue_step(bpe_cuda_ctx *c, u32 z, u64 n_upper, bool encode, bool census, bool ranged, bool sparse, u64 z_ub = 0)
 {
     if (z_ub < z)
         z_ub = z;
@@ -817,7 +825,16 @@ static int enqueue_step(bpe_cuda_ctx *c, u32 z, u64 n_upper, bool encode, bool c
         c->stats.census_runs++;
     }
     const bool hist = ((int)z + 1 <= c->smem_hist_max_vocab);
-    if (ranged)
+    if (sparse)
+    {
+        // SPARSE stream: lists of the pass's merges, replacements + deltas (reads only), rewrite + creation lists
+        const int g = c->sm_count * 4;
+        sparse_plan_kernel<<<1, 32, 0, c->stream>>>(c->d_st);
+        sparse_scan_kernel<<<g, SPX_THREADS, 0, c->stream>>>(c->d_st, c->d_delta);
+        sparse_write_kernel<<<g, SPX_THREADS, 0, c->stream>>>(c->d_st);
+        c->launches += 2;
+    }
+    else if (ranged)
     {
         // RANGED stream: one CTA per range (a == b runs same_pair_range inside the same kernel)
         // the histogram always gets its full budget: the device may be ahead of this id estimate, or batch merges
@@ -890,7 +907,7 @@ struct BatchPlan
     u64 n_upper = 0;
     u64 margin = 0; // table slots it may claim
     u64 zub0 = 0;   // upper bound of the id created by its first pass (the device may be ahead of z0)
-    bool pending = false, census = false, ranged = false;
+    bool pending = false, census = false, ranged = false, sparse = false;
 };
 
 // table slots a batch of G steps may claim: every replacement creates at most two new pair instances, and a
@@ -920,7 +937,7 @@ static int enqueue_batch(bpe_cuda_ctx *c, const BatchPlan &p, bool encode)
     if (!p.pending && (rc = enqueue_select(c, encode)))
         return rc;
     for (u64 g = 0; g < p.G; g++)
-        if ((rc = enqueue_step(c, (u32)(p.z0 + g), p.n_upper, encode, p.census, p.ranged, p.zub0 + (g + 1) * eff_batch(c))))
+        if ((rc = enqueue_step(c, (u32)(p.z0 + g), p.n_upper, encode, p.census, p.ranged, p.sparse, p.zub0 + (g + 1) * eff_batch(c))))
             return rc;
     CU(cudaGetLastError());
     return 0;
@@ -939,6 +956,156 @@ static int poll_wait(bpe_cuda_ctx *c, int slot)
     CU(cudaEventSynchronize(c->poll_ev[slot]));
     c->h_st = c->h_buf[slot];
     return check_state(c);
+}
+
+// ---- LAYOUT_SPARSE (bpe_sparse.cuh) --------------------------------------------------------------------------------
+// A one-GPU run switches to the sparse layout once a pass replaces less than 1/SPARSE_RATIO of the stream: from there
+// on a pass costs in proportion to the occurrences it checks, while a streaming pass reads and writes the whole stream.
+constexpr u64 SPARSE_RATIO = 1000;
+
+struct SparsePtrs
+{
+    u32 *slen, *cl_off, *cl_cnt, *pool, *ipos;
+    const u64 *ikey;
+    const u32 *ioff;
+    u64 *pass_buf;
+    u64 icap, n0;
+    u32 zsw;
+    bool index; // the frozen index and the pools are set too (a switch), not only the vocabulary arrays
+};
+__global__ void sparse_setup_kernel(DevState *st, SparsePtrs q)
+{
+    st->slen = q.slen;
+    st->cl_off = q.cl_off;
+    st->cl_cnt = q.cl_cnt;
+    if (q.index)
+    {
+        st->pool = q.pool;
+        st->ipos = q.ipos;
+        st->ikey = q.ikey;
+        st->ioff = q.ioff;
+        st->pass_buf = q.pass_buf;
+        st->icap = q.icap;
+        st->n0 = q.n0;
+        st->zsw = q.zsw;
+    }
+}
+
+static SparsePtrs sparse_ptrs(const bpe_cuda_ctx *c, bool index)
+{
+    SparsePtrs q{c->d_slen, c->d_cl_off, c->d_cl_cnt, c->d_pool, c->d_ipos, c->d_ikey, c->d_ioff, c->d_pass_buf, 0, 0, 0, index};
+    return q;
+}
+
+template <class T> static int sp_alloc(T *&p, size_t &cap, size_t need)
+{
+    if (need <= cap)
+        return 0;
+    CU(cudaFree(p));
+    p = nullptr;
+    cap = 0;
+    CU(cudaMalloc(&p, need * sizeof(T)));
+    cap = need;
+    return 0;
+}
+
+// byte length, creation-list offset and count per id, for ids below `need` (contents kept; the stream is idle)
+static int sparse_vocab(bpe_cuda_ctx *c, size_t need)
+{
+    if (need <= c->sp_vcap)
+        return 0;
+    const size_t cap = std::max<size_t>(2 * need, 65536);
+    u32 **arr[3] = {&c->d_slen, &c->d_cl_off, &c->d_cl_cnt};
+    for (u32 **a : arr)
+    {
+        u32 *p = nullptr;
+        CU(cudaMalloc(&p, cap * sizeof(u32)));
+        CU(cudaMemsetAsync(p, 0, cap * sizeof(u32), c->stream));
+        if (*a)
+            CU(cudaMemcpyAsync(p, *a, c->sp_vcap * sizeof(u32), cudaMemcpyDeviceToDevice, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+        CU(cudaFree(*a));
+        *a = p;
+    }
+    c->sp_vcap = cap;
+    sparse_setup_kernel<<<1, 1, 0, c->stream>>>(c->d_st, sparse_ptrs(c, false));
+    c->launches++;
+    return 0;
+}
+
+// DENSE -> SPARSE, with a fresh frozen index and empty creation lists.  The stream is idle and c->h_st current.
+static int to_sparse(bpe_cuda_ctx *c)
+{
+    const DevState *h = c->h_st;
+    const u64 n = h->n, n0 = c->stats.n_input, md = h->merges_done, icap = c->tcap;
+    const size_t batch = (size_t)std::max(1, c->batch_steps);
+    int rc;
+    if ((rc = sparse_vocab(c, 256 + md + 3 * batch * eff_batch(c) + 64)))
+        return rc;
+    // byte lengths of every id so far, from the merge log
+    std::vector<u32> pairs(2 * md), len(256 + md);
+    if (md)
+        CU(cudaMemcpy(pairs.data(), c->d_merges, 2 * md * sizeof(u32), cudaMemcpyDeviceToHost));
+    for (u64 t = 0; t < 256; t++)
+        len[t] = 1;
+    for (u64 k = 0; k < md; k++)
+    {
+        const u32 a = pairs[2 * k], b = pairs[2 * k + 1];
+        len[256 + k] = (a < 256 + k ? len[a] : 0) + (b < 256 + k ? len[b] : 0);
+    }
+    CU(cudaMemcpy(c->d_slen, len.data(), len.size() * sizeof(u32), cudaMemcpyHostToDevice));
+    CU(cudaMemsetAsync(c->d_cl_cnt, 0, c->sp_vcap * sizeof(u32), c->stream));
+    const u64 nt = (n + SPX_TILE - 1) / SPX_TILE, it = (icap + 1 + SPX_TILE - 1) / SPX_TILE, ct = (n0 + SPX_TILE - 1) / SPX_TILE;
+    if ((rc = sp_alloc(c->d_ikey, c->ikey_cap, icap)) || (rc = sp_alloc(c->d_icur, c->icur_cap, icap)) ||
+        (rc = sp_alloc(c->d_ioff, c->ioff_cap, icap + 1)) || (rc = sp_alloc(c->d_ipos, c->ipos_cap, n + 1)) ||
+        (rc = sp_alloc(c->d_pool, c->pool_cap, n + 1)) || (rc = sp_alloc(c->d_pass_buf, c->pass_cap, n + 1)) ||
+        (rc = sp_alloc(c->d_sp_tsum, c->sp_tsum_cap, (size_t)(std::max(nt, ct) + it + 2))))
+        return rc;
+    u32 *tsum_tok = c->d_sp_tsum, *tsum_idx = c->d_sp_tsum + std::max(nt, ct) + 1;
+    CU(cudaMemcpyAsync(c->d_ikey, c->d_tkey, icap * sizeof(u64), cudaMemcpyDeviceToDevice, c->stream));
+    CU(cudaMemsetAsync(c->d_ioff, 0, (icap + 1) * sizeof(u32), c->stream));
+    CU(cudaMemsetAsync(c->d_icur, 0, icap * sizeof(u32), c->stream));
+    // the buffer the sparse tokens go to: the one the dense stream is not in, all SENT
+    u32 *x = h->tok[h->cur];
+    u32 *y_alloc = (c->d_tok_alloc[0] + 4 == x) ? c->d_tok_alloc[1] : c->d_tok_alloc[0];
+    CU(cudaMemsetAsync(y_alloc, 0xFF, c->tok_cap * sizeof(u32), c->stream));
+    SparsePtrs q = sparse_ptrs(c, true);
+    q.icap = icap;
+    q.n0 = n0;
+    q.zsw = h->pending ? h->z : (u32)(256 + md);
+    sparse_setup_kernel<<<1, 1, 0, c->stream>>>(c->d_st, q);
+    sparse_count_kernel<<<(unsigned)nt, SPX_THREADS, 0, c->stream>>>(c->d_st, tsum_tok, c->d_ioff);
+    spx_top_scan_kernel<<<1, 1024, 0, c->stream>>>(tsum_tok, (u32)nt);
+    spx_tile_sums_kernel<<<(unsigned)it, SPX_THREADS, 0, c->stream>>>(c->d_ioff, icap + 1, tsum_idx);
+    spx_top_scan_kernel<<<1, 1024, 0, c->stream>>>(tsum_idx, (u32)it);
+    spx_apply_scan_kernel<<<(unsigned)it, SPX_THREADS, 0, c->stream>>>(c->d_ioff, c->d_ioff, icap + 1, tsum_idx);
+    sparse_scatter_kernel<<<(unsigned)nt, SPX_THREADS, 0, c->stream>>>(c->d_st, tsum_tok, c->d_icur);
+    sparse_start_kernel<<<c->sm_count * 8, SPX_THREADS, 0, c->stream>>>(c->d_st);
+    sparse_enter_kernel<<<1, 1, 0, c->stream>>>(c->d_st);
+    c->launches += 9;
+    CU(cudaGetLastError());
+    return poll_state(c);
+}
+
+// SPARSE -> DENSE (the live starts in byte order), before anything that needs positions in one array
+static int to_dense(bpe_cuda_ctx *c)
+{
+    const u64 n0 = c->stats.n_input, ct = (n0 + SPX_TILE - 1) / SPX_TILE;
+    sparse_live_count_kernel<<<(unsigned)ct, SPX_THREADS, 0, c->stream>>>(c->d_st, c->d_sp_tsum);
+    spx_top_scan_kernel<<<1, 1024, 0, c->stream>>>(c->d_sp_tsum, (u32)ct);
+    sparse_compact_kernel<<<(unsigned)ct, SPX_THREADS, 0, c->stream>>>(c->d_st, c->d_sp_tsum);
+    sparse_leave_kernel<<<1, 1, 0, c->stream>>>(c->d_st);
+    c->launches += 4;
+    CU(cudaGetLastError());
+    return 0;
+}
+
+// (the last pass carried nb merges of at most `freq` occurrences each; once sparse, the run stays sparse until
+// something needs a dense stream)
+static bool sparse_wanted(const bpe_cuda_ctx *c, const DevState *h)
+{
+    return c->world == 1 && c->stats.n_input < 0xFFFFFFF0ull &&
+           (h->layout == LAYOUT_SPARSE || (h->merges_done > 0 && (u64)h->freq * std::max<u32>(1, h->nb) * SPARSE_RATIO < h->n));
 }
 
 // Same-bucket ties / exact-threshold iterations / layout changes / candidate rebuilds.
@@ -1065,7 +1232,30 @@ static int run_loop(bpe_cuda_ctx *c, bool encode)
         // The streaming kernel works on the RANGED layout; everything that needs positions in one dense
         // array (static regime, census) keeps the stream dense and uses the general kernel.
         X.ranged = c->want_ranged && !X.census && !h->static_mode && h->n > 0;
-        if (X.ranged && h->layout == LAYOUT_DENSE)
+        // one GPU, late phase: the SPARSE layout
+        X.sparse = X.ranged && sparse_wanted(c, h);
+        if (X.sparse && h->layout != LAYOUT_SPARSE)
+        {
+            if (h->layout == LAYOUT_RANGED)
+            {
+                repack_kernel<<<RANGE_MAX, 1024, 0, c->stream>>>(c->d_st);
+                c->launches++;
+                if ((rc = poll_state(c)))
+                    return rc;
+            }
+            if ((rc = to_sparse(c)))
+                return rc;
+            h = c->h_st;
+        }
+        else if (!X.sparse && h->layout == LAYOUT_SPARSE)
+        {
+            if ((rc = to_dense(c)) || (rc = poll_state(c)))
+                return rc;
+            h = c->h_st;
+        }
+        if (X.sparse && (rc = sparse_vocab(c, (size_t)(z_ub + 3 * batch * bm + 64))))
+            return rc;
+        if (X.ranged && !X.sparse && h->layout == LAYOUT_DENSE)
         {
             partition_kernel<<<1, RANGE_MAX, 0, c->stream>>>(c->d_st);
             c->launches++;
@@ -1096,10 +1286,13 @@ static int run_loop(bpe_cuda_ctx *c, bool encode)
             Y.n_upper = X.n_upper;
             Y.census = false;
             Y.ranged = X.ranged;
+            Y.sparse = X.sparse;
             const bool spec = Y.G > 0 && !X.census && !stat && !prev->static_mode &&
                               (encode || prev->n_global >= STATIC_LIMIT) &&
                               occ_bound + Y.margin <= c->tcap / 2 + c->tcap / 8 &&
-                              delta_need(c, z_ub + Y.G * bm + 2) <= c->delta_cap && m_ub + Y.G * bm + 2 <= c->merges_cap;
+                              delta_need(c, z_ub + Y.G * bm + 2) <= c->delta_cap && m_ub + Y.G * bm + 2 <= c->merges_cap &&
+                              (!X.sparse || z_ub + Y.G * bm + 2 <= c->sp_vcap) &&
+                              !(X.ranged && !X.sparse && sparse_wanted(c, prev)); // (back to the top to switch)
             if (spec)
             {
                 if ((rc = enqueue_batch(c, Y, encode)))
@@ -1136,6 +1329,11 @@ static int run_loop(bpe_cuda_ctx *c, bool encode)
         c->launches++;
         CU(cudaGetLastError());
         if ((rc = poll_state(c)))
+            return rc;
+    }
+    else if (c->h_st->layout == LAYOUT_SPARSE)
+    {
+        if ((rc = to_dense(c)) || (rc = poll_state(c)))
             return rc;
     }
     return 0;
@@ -1381,6 +1579,7 @@ static int run_common(bpe_cuda_ctx *c, u64 max_merges, const bpe_pair_t *enc_mer
     c->stats.final_distinct = (u64)h->distinct;
     c->stats.batch_merges = h->batch_merges;
     c->stats.batch_passes = h->batch_passes;
+    c->stats.sparse_passes = h->sparse_passes;
     c->stats.kernel_launches = c->launches;
     c->stats.ms_device = ms;
     for (int t = 0; t < REF_THREADS; t++)
@@ -1390,16 +1589,21 @@ static int run_common(bpe_cuda_ctx *c, u64 max_merges, const bpe_pair_t *enc_mer
     {
         std::vector<u64> nh(h->merges_done);
         CU(cudaMemcpy(nh.data(), c->d_nhist, h->merges_done * sizeof(u64), cudaMemcpyDeviceToHost));
-        u64 bytes = 0;
+        // (a SPARSE pass counts what it read and wrote: sparse_bytes, summed on the device)
+        u64 bytes = h->sparse_bytes;
         // one pass per entry that is not marked "rode along in a batch"
         std::vector<u64> pass_n;
+        std::vector<bool> pass_sparse;
         for (u64 k = 0; k < h->merges_done; k++)
             if (nh[k] != ~0ull)
-                pass_n.push_back(nh[k]);
+            {
+                pass_n.push_back(nh[k] & ~SPARSE_PASS_MARK);
+                pass_sparse.push_back((nh[k] & SPARSE_PASS_MARK) != 0);
+            }
         for (size_t k = 0; k < pass_n.size(); k++)
         {
             const u64 nk = pass_n[k], nk1 = (k + 1 < pass_n.size()) ? pass_n[k + 1] : c->stats.n_tokens;
-            if (!encode || nk1 != nk)
+            if (!pass_sparse[k] && (!encode || nk1 != nk))
                 bytes += 4 * (nk + nk1);
         }
         c->stats.replace_passes = pass_n.size();
@@ -1587,6 +1791,8 @@ static int resolve_pause(bpe_cuda_ctx *c, bool encode)
         repack_kernel<<<RANGE_MAX, 1024, 0, c->stream>>>(c->d_st);
         c->launches++;
     }
+    else if (h->layout == LAYOUT_SPARSE && (rc = to_dense(c)))
+        return rc;
     if (pause & PAUSE_STATIC)
     {
         // the select kernel latched static_mode; several GPUs: from here on every rank works on the whole stream;
@@ -1656,7 +1862,7 @@ static int resolve_pause(bpe_cuda_ctx *c, bool encode)
     resolver_commit_kernel<<<1, 1, 0, c->stream>>>(c->d_st, c->d_rs);
     c->launches += 9;
     CU(cudaGetLastError());
-    return enqueue_step(c, (u32)(256 + merges_done), n, encode, false, false);
+    return enqueue_step(c, (u32)(256 + merges_done), n, encode, false, false, false);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1755,6 +1961,9 @@ void bpe_cuda_ctx_destroy(bpe_cuda_ctx_t *c)
     for (auto &e : c->prof)
         cudaEventDestroy(e);
     cudaFree(c->d_bytes);
+    for (void *p : {(void *)c->d_ikey, (void *)c->d_ioff, (void *)c->d_icur, (void *)c->d_ipos, (void *)c->d_pool,
+                    (void *)c->d_sp_tsum, (void *)c->d_pass_buf, (void *)c->d_slen, (void *)c->d_cl_off, (void *)c->d_cl_cnt})
+        cudaFree(p);
     cudaFree(c->d_tok_alloc[0]);
     cudaFree(c->d_tok_alloc[1]);
     cudaFree(c->d_st);

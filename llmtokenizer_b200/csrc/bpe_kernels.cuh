@@ -55,8 +55,10 @@ enum : u32
 enum : u32
 {
     LAYOUT_DENSE = 0,
-    LAYOUT_RANGED = 1
+    LAYOUT_RANGED = 1,
+    LAYOUT_SPARSE = 2 // one GPU, late phase: tokens at their byte offsets, never compacted (bpe_sparse.cuh)
 };
+constexpr u64 SPARSE_PASS_MARK = 1ull << 63; // n_hist[k] of a merge whose pass ran on the SPARSE layout
 constexpr int RANGE_MAX = 320;  // ranges per shard (= CTAs of the streaming kernel)
 constexpr int EDGE_WORDS = 8;   // per range: [0..2] first three tokens, [3] second to last, [4] last (SENT where absent)
 enum : u32
@@ -166,6 +168,24 @@ struct DevState
     const u32 *enc_merges;
     u64 enc_total;
     u64 ranks_applied;
+    // LAYOUT_SPARSE (bpe_sparse.cuh): tok[0] == tok[1] holds the id that starts at each byte offset (SENT at every
+    // other byte), start_of[e] the start of the token whose last byte is e; slen = byte length per id
+    u32 *start_of;
+    u32 *slen;
+    u64 n0;      // byte positions of the sparse stream
+    u32 zsw;     // ids below zsw existed when the frozen index was built
+    u32 sp_done; // blocks of sparse_write_kernel that have finished
+    const u64 *ikey; // frozen index: copy of the table keys at the switch, per slot its positions ipos[ioff[s] ..]
+    u64 icap;
+    const u32 *ioff;
+    u32 *ipos;
+    u32 *cl_off, *cl_cnt, *pool; // creation lists: positions where id z was written, pool[cl_off[z] ..][cl_cnt[z]]
+    u64 pool_top, sp_base;
+    u64 *pass_buf;               // replacements of the current pass: position | merge index << 32
+    u32 pass_cnt, pad_pc;
+    u32 sp_cnt[BATCH_MAX], sp_cur[BATCH_MAX], sp_len[BATCH_MAX], sp_kind[BATCH_MAX];
+    const u32 *sp_src[BATCH_MAX];
+    u64 sparse_passes, sparse_bytes;
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -369,6 +389,23 @@ __device__ inline void stream_ends(const DevState *st, u32 buf, u32 layout, u64 
         e.first[k] = SENT;
     e.last2[0] = e.last2[1] = SENT;
     const u32 *t = st->tok[buf];
+    if (layout == LAYOUT_SPARSE)
+    {
+        u64 p = 0;
+        for (int k = 0; k < 3 && p < st->n0; k++)
+        {
+            e.first[k] = t[p];
+            p += st->slen[t[p]];
+        }
+        if (n >= 1)
+        {
+            const u32 lp = st->start_of[st->n0 - 1];
+            e.last2[1] = t[lp];
+            if (n >= 2)
+                e.last2[0] = t[st->start_of[lp - 1]];
+        }
+        return;
+    }
     if (layout == LAYOUT_DENSE)
     {
         for (u64 k = 0; k < 3 && k < n; k++)
