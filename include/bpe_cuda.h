@@ -75,6 +75,11 @@ typedef struct
     uint64_t batch_merges;     /* merges that rode along in another merge's pass                       */
     uint64_t batch_passes;     /* passes that carried more than one merge                              */
     uint64_t sparse_passes;    /* passes that ran on the sparse (byte-anchored, occurrence-indexed) layout */
+    /* only when profiling is enabled: replace_ms = dense_pass_ms + sparse_scan_ms (a sparse pass rewrites the stream
+     * inside the delta application, apply_ms), and the conversions to and from the sparse layout */
+    double sparse_scan_ms, dense_pass_ms, convert_ms;
+    uint64_t sparse_entries;   /* occurrence-list entries the sparse passes checked against the stream        */
+    uint64_t sparse_replacements; /* pair instances the sparse passes replaced                                */
 } bpe_cuda_stats_t;
 
 #define BPE_CUDA_OK 0

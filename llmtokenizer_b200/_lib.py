@@ -18,7 +18,9 @@ class Stats(C.Structure):
         "census_runs", "table_rehashes", "table_capacity", "final_distinct", "kernel_launches", "replace_launches",
         "replace_bytes")] + [(n, C.c_double) for n in ("replace_ms", "ms_device", "ms_h2d", "ms_d2h", "ms_total")] + [
         ("worker_buckets", C.c_uint64 * 16)] + [(n, C.c_double) for n in ("select_ms", "apply_ms", "gap_ms")] + [
-        (n, C.c_uint64) for n in ("replace_passes", "batch_merges", "batch_passes", "sparse_passes")]
+        (n, C.c_uint64) for n in ("replace_passes", "batch_merges", "batch_passes", "sparse_passes")] + [
+        (n, C.c_double) for n in ("sparse_scan_ms", "dense_pass_ms", "convert_ms")] + [
+        (n, C.c_uint64) for n in ("sparse_entries", "sparse_replacements")]
 
     def as_dict(self):
         d = {n: getattr(self, n) for n, _ in self._fields_ if n != "worker_buckets"}

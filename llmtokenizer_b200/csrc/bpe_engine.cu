@@ -258,7 +258,7 @@ struct bpe_cuda_ctx
     // LAYOUT_SPARSE (bpe_sparse.cuh): frozen pair index, creation lists, byte length per id, scan scratch
     u64 *d_ikey = nullptr;
     u32 *d_ioff = nullptr, *d_icur = nullptr, *d_ipos = nullptr, *d_pool = nullptr, *d_sp_tsum = nullptr;
-    u64 *d_pass_buf = nullptr;
+    u32 *d_pass_buf = nullptr;
     size_t ikey_cap = 0, icur_cap = 0, ioff_cap = 0, ipos_cap = 0, pool_cap = 0, pass_cap = 0, sp_tsum_cap = 0;
     u32 *d_slen = nullptr, *d_cl_off = nullptr, *d_cl_cnt = nullptr;
     size_t sp_vcap = 0;
@@ -673,13 +673,17 @@ static cudaError_t launch_chained(bpe_cuda_ctx *c, void (*kernel)(KArgs...), int
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 
-// profiling marks: the interval that ends at a mark is charged to the mark's class
+// profiling marks: the interval that ends at a mark is charged to the mark's class (replace_ms is the sum of the
+// two pass classes)
 enum
 {
     PT_GAP = 0,
     PT_SELECT = 1,
-    PT_REPLACE = 2,
-    PT_APPLY = 3
+    PT_DENSE_PASS = 2,
+    PT_APPLY = 3,
+    PT_SP_SCAN = 4,
+    PT_CONVERT = 5,
+    PT_CLASSES = 6
 };
 static inline void prof_mark(bpe_cuda_ctx *c, int tag)
 {
@@ -827,12 +831,10 @@ static int enqueue_step(bpe_cuda_ctx *c, u32 z, u64 n_upper, bool encode, bool c
     const bool hist = ((int)z + 1 <= c->smem_hist_max_vocab);
     if (sparse)
     {
-        // SPARSE stream: lists of the pass's merges, replacements + deltas (reads only), rewrite + creation lists
-        const int g = c->sm_count * 4;
-        sparse_plan_kernel<<<1, 32, 0, c->stream>>>(c->d_st);
-        sparse_scan_kernel<<<g, SPX_THREADS, 0, c->stream>>>(c->d_st, c->d_delta);
-        sparse_write_kernel<<<g, SPX_THREADS, 0, c->stream>>>(c->d_st);
-        c->launches += 2;
+        // SPARSE stream: lists of the pass's merges, replacements + deltas (reads only); the rewrite and the creation
+        // lists go with the delta application below
+        CU(launch_chained(c, sparse_scan_kernel, c->sm_count * 4, SPX_THREADS, 0, c->d_st, c->d_delta));
+        prof_mark(c, PT_SP_SCAN);
     }
     else if (ranged)
     {
@@ -861,7 +863,8 @@ static int enqueue_step(bpe_cuda_ctx *c, u32 z, u64 n_upper, bool encode, bool c
         else
             replace_kernel<false><<<grid, R_THREADS, smem, c->stream>>>(c->d_st, c->d_desc, c->d_pdesc, c->d_delta);
     }
-    prof_mark(c, PT_REPLACE);
+    if (!sparse)
+        prof_mark(c, PT_DENSE_PASS);
     c->launches++;
     c->stats.replace_launches++;
     // every thread looks at one token's four counters (128 bits) per trip; 32 blocks keep the "last block" wait short
@@ -968,7 +971,7 @@ struct SparsePtrs
     u32 *slen, *cl_off, *cl_cnt, *pool, *ipos;
     const u64 *ikey;
     const u32 *ioff;
-    u64 *pass_buf;
+    u32 *pass_buf;
     u64 icap, n0;
     u32 zsw;
     bool index; // the frozen index and the pools are set too (a switch), not only the vocabulary arrays
@@ -1040,6 +1043,7 @@ static int to_sparse(bpe_cuda_ctx *c)
     const u64 n = h->n, n0 = c->stats.n_input, md = h->merges_done, icap = c->tcap;
     const size_t batch = (size_t)std::max(1, c->batch_steps);
     int rc;
+    prof_mark(c, PT_GAP);
     if ((rc = sparse_vocab(c, 256 + md + 3 * batch * eff_batch(c) + 64)))
         return rc;
     // byte lengths of every id so far, from the merge log
@@ -1058,7 +1062,7 @@ static int to_sparse(bpe_cuda_ctx *c)
     const u64 nt = (n + SPX_TILE - 1) / SPX_TILE, it = (icap + 1 + SPX_TILE - 1) / SPX_TILE, ct = (n0 + SPX_TILE - 1) / SPX_TILE;
     if ((rc = sp_alloc(c->d_ikey, c->ikey_cap, icap)) || (rc = sp_alloc(c->d_icur, c->icur_cap, icap)) ||
         (rc = sp_alloc(c->d_ioff, c->ioff_cap, icap + 1)) || (rc = sp_alloc(c->d_ipos, c->ipos_cap, n + 1)) ||
-        (rc = sp_alloc(c->d_pool, c->pool_cap, n + 1)) || (rc = sp_alloc(c->d_pass_buf, c->pass_cap, n + 1)) ||
+        (rc = sp_alloc(c->d_pool, c->pool_cap, n + 1)) || (rc = sp_alloc(c->d_pass_buf, c->pass_cap, 2 * n + 2)) ||
         (rc = sp_alloc(c->d_sp_tsum, c->sp_tsum_cap, (size_t)(std::max(nt, ct) + it + 2))))
         return rc;
     u32 *tsum_tok = c->d_sp_tsum, *tsum_idx = c->d_sp_tsum + std::max(nt, ct) + 1;
@@ -1082,6 +1086,7 @@ static int to_sparse(bpe_cuda_ctx *c)
     sparse_scatter_kernel<<<(unsigned)nt, SPX_THREADS, 0, c->stream>>>(c->d_st, tsum_tok, c->d_icur);
     sparse_start_kernel<<<c->sm_count * 8, SPX_THREADS, 0, c->stream>>>(c->d_st);
     sparse_enter_kernel<<<1, 1, 0, c->stream>>>(c->d_st);
+    prof_mark(c, PT_CONVERT);
     c->launches += 9;
     CU(cudaGetLastError());
     return poll_state(c);
@@ -1091,10 +1096,12 @@ static int to_sparse(bpe_cuda_ctx *c)
 static int to_dense(bpe_cuda_ctx *c)
 {
     const u64 n0 = c->stats.n_input, ct = (n0 + SPX_TILE - 1) / SPX_TILE;
+    prof_mark(c, PT_GAP);
     sparse_live_count_kernel<<<(unsigned)ct, SPX_THREADS, 0, c->stream>>>(c->d_st, c->d_sp_tsum);
     spx_top_scan_kernel<<<1, 1024, 0, c->stream>>>(c->d_sp_tsum, (u32)ct);
     sparse_compact_kernel<<<(unsigned)ct, SPX_THREADS, 0, c->stream>>>(c->d_st, c->d_sp_tsum);
     sparse_leave_kernel<<<1, 1, 0, c->stream>>>(c->d_st);
+    prof_mark(c, PT_CONVERT);
     c->launches += 4;
     CU(cudaGetLastError());
     return 0;
@@ -1605,23 +1612,29 @@ static int run_common(bpe_cuda_ctx *c, u64 max_merges, const bpe_pair_t *enc_mer
             const u64 nk = pass_n[k], nk1 = (k + 1 < pass_n.size()) ? pass_n[k + 1] : c->stats.n_tokens;
             if (!pass_sparse[k] && (!encode || nk1 != nk))
                 bytes += 4 * (nk + nk1);
+            if (pass_sparse[k])
+                c->stats.sparse_replacements += nk - nk1; // (a replacement removes one token)
         }
         c->stats.replace_passes = pass_n.size();
         c->stats.replace_bytes = bytes;
     }
+    c->stats.sparse_entries = h->sparse_entries;
     if (c->profile_replace)
     {
-        double tot[4] = {0, 0, 0, 0};
+        double tot[PT_CLASSES] = {};
         for (size_t i = 0; i + 1 < c->prof_used; i++)
         {
             float e = 0;
             CU(cudaEventElapsedTime(&e, c->prof[i], c->prof[i + 1]));
-            tot[c->prof_tag[i + 1] & 3] += e;
+            tot[c->prof_tag[i + 1]] += e;
         }
         c->stats.gap_ms = tot[PT_GAP];
         c->stats.select_ms = tot[PT_SELECT];
-        c->stats.replace_ms = tot[PT_REPLACE];
         c->stats.apply_ms = tot[PT_APPLY];
+        c->stats.dense_pass_ms = tot[PT_DENSE_PASS];
+        c->stats.sparse_scan_ms = tot[PT_SP_SCAN];
+        c->stats.convert_ms = tot[PT_CONVERT];
+        c->stats.replace_ms = tot[PT_DENSE_PASS] + tot[PT_SP_SCAN];
     }
     c->stats.ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (stats_out)

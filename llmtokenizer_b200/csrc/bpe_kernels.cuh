@@ -174,18 +174,20 @@ struct DevState
     u32 *slen;
     u64 n0;      // byte positions of the sparse stream
     u32 zsw;     // ids below zsw existed when the frozen index was built
-    u32 sp_done; // blocks of sparse_write_kernel that have finished
     const u64 *ikey; // frozen index: copy of the table keys at the switch, per slot its positions ipos[ioff[s] ..]
     u64 icap;
     const u32 *ioff;
     u32 *ipos;
     u32 *cl_off, *cl_cnt, *pool; // creation lists: positions where id z was written, pool[cl_off[z] ..][cl_cnt[z]]
-    u64 pool_top, sp_base;
-    u64 *pass_buf;               // replacements of the current pass: position | merge index << 32
-    u32 pass_cnt, pad_pc;
-    u32 sp_cnt[BATCH_MAX], sp_cur[BATCH_MAX], sp_len[BATCH_MAX], sp_kind[BATCH_MAX];
-    const u32 *sp_src[BATCH_MAX];
+    u64 pool_top;
+    // replacements of the current pass, merge by merge: merge i's sp_cnt[i] positions at pass_buf[sp_ent[i] ..], where
+    // sp_ent[i] is the number of list entries of the merges before it (a merge replaces at most one pair instance per
+    // entry, and the lists of one pass are disjoint: the frozen lists of different pairs and the creation lists of
+    // different ids; so 2 n + 2 words hold any pass)
+    u32 *pass_buf;
+    u32 sp_cnt[BATCH_MAX], sp_ent[BATCH_MAX];
     u64 sparse_passes, sparse_bytes;
+    u64 sparse_entries; // list entries the sparse scans checked
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -1862,11 +1864,69 @@ __device__ __noinline__ void apply_deltas(DevState *st, int32_t *delta, u32 gtid
     }
 }
 
-// the pass is over: its output becomes the current stream (one thread, after every delta is applied)
+// LAYOUT_SPARSE (bpe_sparse.cuh): the write half of a pass, run by the blocks that apply its deltas (the scan that
+// recorded the replacements in pass_buf is complete, and the table and the stream are disjoint).  Every block calls it.
+// Replacement r of the pass (counted merge by merge) goes to pool[pool_top + r]: the creation list of z + i is
+// pool[pool_top + sum of sp_cnt[j < i] ..], as finish_pass records it.
+__device__ inline void sparse_rewrite(DevState *st, u32 gtid, u32 gsize)
+{
+    __shared__ u32 s_la[BATCH_MAX], s_lb[BATCH_MAX], s_ent[BATCH_MAX], s_cum[BATCH_MAX + 1];
+    const u32 nb = st->nb, z = st->z;
+    u32 *tok = st->tok[st->cur], *so = st->start_of, *pool = st->pool + st->pool_top;
+    if (threadIdx.x == 0)
+    {
+        u32 r = 0;
+        for (u32 i = 0; i < nb; i++)
+        {
+            s_la[i] = st->slen[st->ba[i]];
+            s_lb[i] = st->slen[st->bb[i]];
+            s_ent[i] = st->sp_ent[i];
+            s_cum[i] = r;
+            r += st->sp_cnt[i];
+        }
+        s_cum[nb] = r;
+    }
+    __syncthreads();
+    const u32 total = s_cum[nb];
+    for (u32 r = gtid; r < total; r += gsize)
+    {
+        u32 i = 0;
+        while (r >= s_cum[i + 1])
+            i++;
+        const u32 p = st->pass_buf[s_ent[i] + (r - s_cum[i])];
+        const u32 q = p + s_la[i];
+        tok[p] = z + i;
+        tok[q] = SENT;
+        so[q + s_lb[i] - 1] = p;
+        pool[r] = p;
+    }
+}
+
+// the pass is over: its output becomes the current stream (one thread, after every delta is applied - and on the
+// sparse layout, after the whole grid has rewritten the stream)
 __device__ __forceinline__ void finish_pass(DevState *st)
 {
     if (!st->skip)
     {
+        if (st->layout == LAYOUT_SPARSE)
+        {
+            // the creation lists of the new ids, and the counters the next pass's scan adds to back at zero
+            const u32 nb = st->nb, z = st->z;
+            u64 top = st->pool_top, r = 0;
+            for (u32 i = 0; i < nb; i++)
+            {
+                const u32 c = st->sp_cnt[i];
+                st->cl_off[z + i] = (u32)top;
+                st->cl_cnt[z + i] = c;
+                top += c;
+                r += c;
+                st->sp_cnt[i] = 0;
+            }
+            st->pool_top = top;
+            st->sparse_passes++;
+            st->n_hist[st->merges_done - nb] |= SPARSE_PASS_MARK;
+            st->n_next = st->n - r; // every replacement removes one token
+        }
         st->n = st->n_next;
         st->cur ^= 1u;
         st->layout = st->layout_next;
@@ -1879,6 +1939,8 @@ __global__ void __launch_bounds__(256) apply_kernel(DevState *st, int32_t *delta
 {
     if (st->stop != STOP_RUN || !st->pending)
         return;
+    if (!st->skip && st->layout == LAYOUT_SPARSE)
+        sparse_rewrite(st, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
     if (!st->skip)
         apply_deltas(st, delta, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
     __syncthreads();
@@ -1922,6 +1984,7 @@ __global__ void __launch_bounds__(SEL_THREADS) apply_select_kernel(DevState *st,
     const u32 world = st->world;
     const bool xch = world > 1 && pending && !st->skip; // this launch carries an exchange
     const u32 seq = st->xseq + (xch ? 1u : 0u);          // the exchange whose records describe the stream from now on
+    const bool sparse = pending && !st->skip && st->layout == LAYOUT_SPARSE; // the apply blocks also rewrite the stream
     const u32 nb_apply = gridDim.x - 1; // the last block of the grid only looks up the stream's last pair
     if (blockIdx.x == nb_apply)
     {
@@ -1949,7 +2012,11 @@ __global__ void __launch_bounds__(SEL_THREADS) apply_select_kernel(DevState *st,
     else if (xch)
         push_deltas(st, delta, blockIdx.x * blockDim.x + threadIdx.x, nb_apply * blockDim.x, seq & 1u);
     else if (pending && !st->skip)
+    {
+        if (sparse)
+            sparse_rewrite(st, blockIdx.x * blockDim.x + threadIdx.x, nb_apply * blockDim.x);
         apply_deltas(st, delta, blockIdx.x * blockDim.x + threadIdx.x, nb_apply * blockDim.x);
+    }
     if (xch)
     {
         __syncthreads();
@@ -1993,7 +2060,7 @@ __global__ void __launch_bounds__(SEL_THREADS) apply_select_kernel(DevState *st,
     if (world > 1 && (blockIdx.x == nb_apply) && threadIdx.x < MAX_RANKS * REC_INTS)
         s_recs[threadIdx.x] = ld_relaxed_sys_u32(xchg_recs(st->x.local, seq & 1u) + threadIdx.x);
     __syncthreads();
-    if (blockIdx.x == nb_apply && threadIdx.x == 0 && mode == AS_TRAIN)
+    if (blockIdx.x == nb_apply && threadIdx.x == 0 && mode == AS_TRAIN && !sparse)
     {
         const bool flip0 = pending && !st->skip;
         const u64 key = last_pair_key(st, s_recs, flip0 ? (st->cur ^ 1u) : st->cur, flip0 ? st->layout_next : st->layout,
@@ -2028,6 +2095,8 @@ __global__ void __launch_bounds__(SEL_THREADS) apply_select_kernel(DevState *st,
         if (pending)
             finish_pass(st);
     }
+    if (sparse)
+        __syncthreads(); // (thread 32 below reads the stream length finish_pass has just set)
     if (mode == AS_APPLY_ONLY)
         return;
     if (encode)
@@ -2038,9 +2107,29 @@ __global__ void __launch_bounds__(SEL_THREADS) apply_select_kernel(DevState *st,
     }
     if (threadIdx.x == 32)
     {
-        // the key and (unless this very apply created it) its slot were looked up while the deltas were applied
-        const u64 key = *reinterpret_cast<volatile u64 *>(&st->probe_key);
-        u64 slot = *reinterpret_cast<volatile u64 *>(&st->probe_slot);
+        // the key and (unless this very apply created it) its slot were looked up while the deltas were applied.
+        // A sparse pass's stream is rewritten by the same blocks that apply the deltas, so the probe block could not
+        // read its last pair; this block can: every other block passed the sel_done handshake after its share of the
+        // rewrite (L2 loads: lines cached in this SM's L1 before the rewrite must not be read).
+        u64 key, slot;
+        if (sparse)
+        {
+            key = EMPTY_KEY;
+            slot = NO_SLOT;
+            if (st->n >= 2)
+            {
+                const u32 *t = st->tok[st->cur], *so = st->start_of;
+                const u32 lp = __ldcg(so + st->n0 - 1);
+                const u32 x = __ldcg(t + __ldcg(so + lp - 1)), y = __ldcg(t + lp);
+                if (x != SENT && y != SENT)
+                    key = (u64)x | ((u64)y << 32);
+            }
+        }
+        else
+        {
+            key = *reinterpret_cast<volatile u64 *>(&st->probe_key);
+            slot = *reinterpret_cast<volatile u64 *>(&st->probe_slot);
+        }
         if (key != EMPTY_KEY && slot == NO_SLOT)
             slot = table_find(st->tkey, st->tcap, key, murmur3_pair((u32)key, (u32)(key >> 32)));
         s_pre.last_new = (key != EMPTY_KEY && slot != NO_SLOT && __ldcg(cnt_ptr(st->tmeta, slot)) == 1u) ? 1u : 0u;

@@ -17,10 +17,11 @@
 // Every entry is checked (tok[p] == a and tok[next(p)] == b), so entries whose token has since been merged away, on
 // either side, are skipped: the replaced right-hand token is overwritten with SENT.
 //
-// A pass is three launches: sparse_plan_kernel (one warp: the lists of the pass's merges), sparse_scan_kernel (checks
-// the entries, finds the replacements and emits exactly the pair-count deltas replace_stream_kernel emits; it reads
-// the stream only) and sparse_write_kernel (rewrites the stream and appends the creation lists).  Splitting the read
-// from the write keeps every neighbour a replacement looks at the one of the stream before the pass.
+// A pass is two launches, both chained with programmatic dependent launch: sparse_scan_kernel (plans the lists of the
+// pass's merges, checks the entries, finds the replacements and emits exactly the pair-count deltas
+// replace_stream_kernel emits; it reads the stream only), then the delta application, whose blocks also rewrite the
+// stream and fill the creation lists (sparse_rewrite, bpe_kernels.cuh).  Splitting the read from the write keeps every
+// neighbour a replacement looks at the one of the stream before the pass.
 namespace bpe
 {
 
@@ -215,6 +216,8 @@ __global__ void sparse_enter_kernel(DevState *st)
     st->tok[0] = st->tok[1] = t;
     st->layout = st->layout_next = LAYOUT_SPARSE;
     st->pool_top = 0;
+    for (int i = 0; i < BATCH_MAX; i++)
+        st->sp_cnt[i] = 0;
 }
 
 // ---- SPARSE -> DENSE: the live starts in byte order ---------------------------------------------------------------
@@ -266,56 +269,6 @@ __global__ void sparse_leave_kernel(DevState *st)
 }
 
 // ---- the pass -----------------------------------------------------------------------------------------------------
-// One warp: for merge i of the pass, where its occurrences are listed.  kind 0: frozen index (positions of a),
-// kind 1: creation list of a, kind 2: creation list of b (positions of b).
-__global__ void sparse_plan_kernel(DevState *st)
-{
-    if (st->stop != STOP_RUN || st->skip)
-        return;
-    const u32 nb = st->nb, i = threadIdx.x;
-    if (i == 0)
-    {
-        st->n_next = st->n;
-        st->layout_next = LAYOUT_SPARSE;
-        st->pass_cnt = 0;
-        st->sp_base = st->pool_top;
-        if (st->a == st->b && nb != 1)
-            atomicOr(&st->err, ERR_PROBE); // a == a passes carry one merge
-    }
-    if (i >= BATCH_MAX)
-        return;
-    st->sp_cnt[i] = 0;
-    st->sp_cur[i] = 0;
-    u32 len = 0, kind = 0;
-    const u32 *src = nullptr;
-    if (i < nb)
-    {
-        const u32 a = st->ba[i], b = st->bb[i], zsw = st->zsw;
-        st->slen[st->z + i] = st->slen[a] + st->slen[b];
-        if (a < zsw && b < zsw)
-        {
-            const u64 slot = table_find(st->ikey, st->icap, (u64)a | ((u64)b << 32), murmur3_pair(a, b));
-            if (slot != NO_SLOT)
-            {
-                src = st->ipos + st->ioff[slot];
-                len = st->ioff[slot + 1] - st->ioff[slot];
-            }
-        }
-        else
-        {
-            const bool ya = a >= zsw, yb = b >= zsw;
-            const u32 ca = ya ? st->cl_cnt[a] : ~0u, cb = yb ? st->cl_cnt[b] : ~0u;
-            kind = (ca <= cb) ? 1u : 2u;
-            const u32 t = (kind == 1) ? a : b;
-            src = st->pool + st->cl_off[t];
-            len = st->cl_cnt[t];
-        }
-    }
-    st->sp_src[i] = src;
-    st->sp_len[i] = len;
-    st->sp_kind[i] = kind;
-}
-
 __device__ __forceinline__ u32 sp_prev_tok(const u32 *tok, const u32 *so, u32 p) { return p ? tok[so[p - 1]] : SENT; }
 
 // one warp-aggregated atomicAdd per distinct address
@@ -332,28 +285,67 @@ __device__ __forceinline__ u32 sp_bump(u32 *ctr)
     return base + (u32)__popc(peers & ((1u << lane) - 1u));
 }
 
+// Where the occurrences of merge i of the pass are listed.  kind 0: frozen index (positions of a), kind 1: creation
+// list of a, kind 2: creation list of b (positions of b).
+__device__ __forceinline__ void sparse_plan(const DevState *st, u32 a, u32 b, const u32 *&src, u32 &len, u32 &kind)
+{
+    const u32 zsw = st->zsw;
+    src = nullptr;
+    len = 0;
+    kind = 0;
+    if (a < zsw && b < zsw)
+    {
+        const u64 slot = table_find(st->ikey, st->icap, (u64)a | ((u64)b << 32), murmur3_pair(a, b));
+        if (slot != NO_SLOT)
+        {
+            src = st->ipos + st->ioff[slot];
+            len = st->ioff[slot + 1] - st->ioff[slot];
+        }
+        return;
+    }
+    const bool ya = a >= zsw, yb = b >= zsw;
+    const u32 ca = ya ? st->cl_cnt[a] : ~0u, cb = yb ? st->cl_cnt[b] : ~0u;
+    kind = (ca <= cb) ? 1u : 2u;
+    const u32 t = (kind == 1) ? a : b;
+    src = st->pool + st->cl_off[t];
+    len = st->cl_cnt[t];
+}
+
+// The first of a sparse pass's two launches (the second, the delta application, rewrites the stream: sparse_rewrite).
+// Every block plans the pass's lists itself (nb probes, L2 hits after the first block), so no launch of its own is
+// needed for that, whichever launch decided the pass.  The counters it adds to (sp_cnt) are zero on entry: finish_pass
+// clears them.
 __global__ void __launch_bounds__(SPX_THREADS) sparse_scan_kernel(DevState *st, int32_t *delta)
 {
+    pdl_wait();
+    pdl_launch_dependents();
     if (st->stop != STOP_RUN || st->skip)
         return;
     __shared__ u32 s_a[BATCH_MAX], s_b[BATCH_MAX], s_la[BATCH_MAX], s_lb[BATCH_MAX], s_len[BATCH_MAX], s_kind[BATCH_MAX];
     __shared__ const u32 *s_src[BATCH_MAX];
-    __shared__ u32 s_pre[BATCH_MAX + 1], s_cnt[BATCH_MAX];
+    __shared__ u32 s_pre[BATCH_MAX + 1];
     __shared__ unsigned long long s_bytes;
     const u32 nb = st->nb, z = st->z, VS = z + nb;
-    const u32 *tok = st->tok[st->cur], *so = st->start_of, *slen = st->slen;
+    const u32 *tok = st->tok[st->cur], *so = st->start_of;
+    u32 *slen = st->slen;
     int32_t *gdelta = delta + HDR_INTS;
     if (threadIdx.x < BATCH_MAX)
     {
         const u32 i = threadIdx.x;
-        s_a[i] = i < nb ? st->ba[i] : SENT;
-        s_b[i] = i < nb ? st->bb[i] : SENT;
-        s_la[i] = i < nb ? slen[s_a[i]] : 0;
-        s_lb[i] = i < nb ? slen[s_b[i]] : 0;
-        s_len[i] = i < nb ? st->sp_len[i] : 0;
-        s_kind[i] = st->sp_kind[i];
-        s_src[i] = st->sp_src[i];
-        s_cnt[i] = 0;
+        const u32 a = i < nb ? st->ba[i] : SENT, b = i < nb ? st->bb[i] : SENT;
+        const u32 *src = nullptr;
+        u32 len = 0, kind = 0;
+        if (i < nb)
+            sparse_plan(st, a, b, src, len, kind);
+        s_a[i] = a;
+        s_b[i] = b;
+        s_la[i] = i < nb ? slen[a] : 0;
+        s_lb[i] = i < nb ? slen[b] : 0;
+        s_len[i] = len;
+        s_kind[i] = kind;
+        s_src[i] = src;
+        if (blockIdx.x == 0 && i < nb)
+            slen[z + i] = s_la[i] + s_lb[i]; // (ids below z only are read in this launch)
     }
     if (threadIdx.x == 0)
         s_bytes = 0;
@@ -367,6 +359,14 @@ __global__ void __launch_bounds__(SPX_THREADS) sparse_scan_kernel(DevState *st, 
             r += s_len[i];
         }
         s_pre[BATCH_MAX] = r;
+        if (blockIdx.x == 0)
+        {
+            for (u32 i = 0; i < nb; i++)
+                st->sp_ent[i] = s_pre[i];
+            st->sparse_entries += r;
+            if (s_a[0] == s_b[0] && nb != 1)
+                atomicOr(&st->err, ERR_PROBE); // a == a passes carry one merge
+        }
     }
     __syncthreads();
     const u32 total = s_pre[BATCH_MAX];
@@ -433,8 +433,7 @@ __global__ void __launch_bounds__(SPX_THREADS) sparse_scan_kernel(DevState *st, 
                         delta_add(st, gdelta, off + (u64)y * 4 + 1, 1);
                     delta_add(st, gdelta, off + (u64)y * 4 + 3, 1);
                 }
-                st->pass_buf[sp_bump(&st->pass_cnt)] = (u64)cur;
-                atomicAdd(&s_cnt[0], 1u);
+                st->pass_buf[s_pre[0] + sp_bump(&st->sp_cnt[0])] = cur;
                 my_bytes += 16 + 8 + 16;
                 first = false;
                 if (!nm)
@@ -475,75 +474,15 @@ __global__ void __launch_bounds__(SPX_THREADS) sparse_scan_kernel(DevState *st, 
             delta_add(st, gdelta, off + (u64)y * 4 + 1, 1);
             delta_add(st, gdelta, off + (u64)y * 4 + 3, 1);
         }
-        st->pass_buf[sp_bump(&st->pass_cnt)] = (u64)p | ((u64)i << 32);
-        atomicAdd(&s_cnt[i], 1u);
+        st->pass_buf[s_pre[i] + sp_bump(&st->sp_cnt[i])] = p;
         my_bytes += 24 + 8 + 16;
     }
-    atomicAdd(&s_bytes, (unsigned long long)my_bytes);
+    if (my_bytes)
+        atomicAdd(&s_bytes, (unsigned long long)my_bytes);
     __syncthreads();
-    if (threadIdx.x < nb && s_cnt[threadIdx.x])
-        atomicAdd(&st->sp_cnt[threadIdx.x], s_cnt[threadIdx.x]);
-    if (threadIdx.x == 0)
-    {
-        u32 r = 0;
-        for (u32 i = 0; i < nb; i++)
-            r += s_cnt[i];
-        if (r)
-            atomicAdd(&st->n_next, (u64)0 - (u64)r);
+    // (a block that checked no entry adds nothing: a pass of a few thousand entries costs a few dozen global atomics)
+    if (threadIdx.x == 0 && s_bytes)
         atomicAdd(&st->sparse_bytes, s_bytes);
-    }
-}
-
-__global__ void __launch_bounds__(SPX_THREADS) sparse_write_kernel(DevState *st)
-{
-    if (st->stop != STOP_RUN || st->skip)
-        return;
-    __shared__ u32 s_la[BATCH_MAX], s_lb[BATCH_MAX], s_off[BATCH_MAX];
-    const u32 nb = st->nb, z = st->z;
-    u32 *tok = st->tok[st->cur], *so = st->start_of;
-    if (threadIdx.x == 0)
-    {
-        u64 r = st->sp_base;
-        for (u32 i = 0; i < nb; i++)
-        {
-            s_la[i] = st->slen[st->ba[i]];
-            s_lb[i] = st->slen[st->bb[i]];
-            s_off[i] = (u32)r;
-            r += st->sp_cnt[i];
-        }
-    }
-    __syncthreads();
-    const u32 total = st->pass_cnt;
-    for (u32 r = blockIdx.x * blockDim.x + threadIdx.x; r < total; r += gridDim.x * blockDim.x)
-    {
-        const u64 rec = st->pass_buf[r];
-        const u32 p = (u32)rec, i = (u32)(rec >> 32);
-        const u32 q = p + s_la[i];
-        tok[p] = z + i;
-        tok[q] = SENT;
-        so[q + s_lb[i] - 1] = p;
-        st->pool[s_off[i] + sp_bump(&st->sp_cur[i])] = p;
-    }
-    __syncthreads();
-    if (threadIdx.x == 0)
-    {
-        __threadfence();
-        if (atomicAdd(&st->sp_done, 1u) == gridDim.x - 1)
-        {
-            st->sp_done = 0;
-            u64 top = st->sp_base;
-            for (u32 i = 0; i < nb; i++)
-            {
-                st->cl_off[z + i] = (u32)top;
-                st->cl_cnt[z + i] = st->sp_cnt[i];
-                top += st->sp_cnt[i];
-            }
-            st->pool_top = top;
-            st->sparse_passes++;
-            const u64 k0 = st->merges_done - nb;
-            st->n_hist[k0] |= SPARSE_PASS_MARK;
-        }
-    }
 }
 
 } // namespace bpe
